@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the Snappy hot path on B200 (BASELINE.json configs[1] and [2]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step is one pass of the hot path over one batch: the 1 GiB synthetic *mixed* corpus
 (text-like / low-entropy / random in 1 MiB segments, SURVEY.md 8d) per GPU.
@@ -23,6 +23,12 @@ barrier and the max-over-ranks of the timings.
 
 `--impl reference` times the reference's own CPU implementation (all host cores) on a bounded
 sample of the same workload and prints the same JSON line with "impl": "reference".
+
+`--dump-outputs DIR` writes, on rank 0, what each timed device leg returned in its last step
+(decompress: output bytes + block offsets; compress and BST: stream + block offsets) as
+DIR/<leg>_<array>.npy, so that two builds can be compared output for output on the same seeded
+inputs.  Byte arrays are stored as float32 values at fixed, seeded positions (<leg>_<array>_sample)
+plus float64 byte sums of every 64 KiB chunk (<leg>_<array>_chunk_sums); offsets as float64.
 """
 from __future__ import annotations
 
@@ -44,6 +50,9 @@ GIB = 1 << 30
 SEED = 20261018
 METRIC = "decompress GB/s (uncompressed)"
 DECODE_KERNEL = "k_decode_seg (+ k_copy_literal_blocks)"
+DUMP_SAMPLE = 1 << 21       # sampled positions per byte array (8 MiB as float32)
+DUMP_MAX_ENTRIES = 1 << 19  # longer offset / chunk-sum arrays are sampled too (4 MiB as float64)
+DUMP_LIMIT = 64 << 20       # all dumped files together
 
 
 # ------------------------------------------------------------------------------ CPU baseline
@@ -150,17 +159,14 @@ def run_reference_arm(args) -> None:
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    t0 = time.time()
-    # a "step" is one bounded sample (16 x 48 MiB shards through the reference, ~10 s); W and K are
-    # capped (1 warm-up, 3 timed) so that the run ends within a few minutes whatever was asked for
+    # a "step" is one bounded sample (16 x 48 MiB shards through the reference, ~10 s); W is capped
+    # at 1 warm-up, K steps are timed as asked
     warm = min(max(args.warmup, 0), 1)
     for _ in range(warm):
         cpu_baseline()
     base = cpu_baseline()
     vals = [base["value"]]
-    for _ in range(max(0, min(args.steps, 3) - 1)):
-        if time.time() - t0 > 150:
-            break
+    for _ in range(args.steps - 1):
         vals.append(cpu_baseline()["value"])
     v = statistics.median(vals)
     base["value"] = v
@@ -171,7 +177,7 @@ def run_reference_arm(args) -> None:
         "config": {"workload": "mixed corpus (text/low-entropy/random, 1 MiB segments), decompression, "
                                "reference CPU build on all host cores; BOUNDED SAMPLE of the GPU arm's 1 GiB workload "
                                "(16 x 48 MiB shards per step, same generator and seed) -- CPU throughput is "
-                               "size-independent, so config and step count differ from the GPU arm by design",
+                               "size-independent, so the config differs from the GPU arm by design",
                    "spread": {"min": min(vals), "max": max(vals), "samples": len(vals)}},
         "cpu_baseline": base,
         "e2e": {"value": v, "unit": "GB/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -229,6 +235,42 @@ def file_layer_e2e(api, data, c_bytes: int) -> dict:
         return out
     finally:
         shutil.rmtree(d, ignore_errors=True)
+
+
+# ------------------------------------------------------------------------------ --dump-outputs
+def _seeded_positions(n: int, k: int):
+    """k sorted positions in [0, n), a function of (SEED, n, k) only; None when n <= k (keep everything)."""
+    import numpy as np
+    if n <= k:
+        return None
+    return np.sort(np.random.default_rng(SEED).integers(0, n, size=k))
+
+
+def _save_values(out_dir: str, name: str, t, k: int, dtype) -> int:
+    import numpy as np
+    import torch
+    pos = _seeded_positions(t.numel(), k)
+    if pos is not None:
+        t = t[torch.from_numpy(pos).to(t.device)]
+    path = os.path.join(out_dir, name + ".npy")
+    np.save(path, t.cpu().numpy().astype(dtype))
+    return os.path.getsize(path)
+
+
+def dump_leg(out_dir: str, leg: str, data_name: str, data, offsets) -> int:
+    """One timed leg's results: a uint8 device tensor (sampled bytes + 64 KiB chunk sums, so that every byte
+    counts) and its block offsets.  Returns the bytes written."""
+    import numpy as np
+    import torch
+    chunk = 1 << 16
+    n = data.numel()
+    full = n // chunk * chunk
+    sums = data[:full].view(-1, chunk).sum(1, dtype=torch.int64)
+    if full < n:
+        sums = torch.cat([sums, data[full:].sum(dtype=torch.int64).view(1)])
+    return (_save_values(out_dir, f"{leg}_{data_name}_sample", data, DUMP_SAMPLE, np.float32)
+            + _save_values(out_dir, f"{leg}_{data_name}_chunk_sums", sums, DUMP_MAX_ENTRIES, np.float64)
+            + _save_values(out_dir, f"{leg}_block_offsets", offsets, DUMP_MAX_ENTRIES, np.float64))
 
 
 # ------------------------------------------------------------------------------ GPU arm
@@ -353,12 +395,19 @@ def run_gpu_arm(args) -> None:
     td = timed(step_decompress, DECODE_KERNEL)
     codec.check_status()
     assert torch.equal(out, data), "round trip failed (pipelined path)"
+    dump_dir = args.dump_outputs if rank == 0 else None
+    dumped = 0
+    if dump_dir:
+        os.makedirs(dump_dir, exist_ok=True)
+        dumped += dump_leg(dump_dir, "decompress", "output", out, k0_index)
     tk = timed(step_decode_kernel, DECODE_KERNEL)
     codec.check_status()
     td["kernel_ms"] = tk["kernel_ms"]
     td["unpipelined_ms_per_step"] = tk["total_ms"] / args.steps
     tc = timed(step_compress, "k_parse_hash_global (+ k_emit + k_scan_sizes + k_gather)")
     codec.check_status()
+    if dump_dir:
+        dumped += dump_leg(dump_dir, "compress", "stream", codec.result_stream(), codec.block_offsets)
 
     # ---- BASELINE configs[3]: the BST (exact-key) path on 1 GiB of low-entropy + random data
     tb = None
@@ -402,6 +451,9 @@ def run_gpu_arm(args) -> None:
         tb = timed(step_bst, "k_parse_exact_global (+ k_emit + k_scan_sizes + k_gather)")
         codec.check_status()
         tb["c_bytes"], tb["parity"], tb["base"] = cb_bytes, bst_parity, base_b
+        if dump_dir:
+            dumped += dump_leg(dump_dir, "bst", "stream", codec.result_stream(), codec.block_offsets)
+    assert dumped <= DUMP_LIMIT, f"--dump-outputs wrote {dumped} bytes, more than {DUMP_LIMIT}"
 
     # ---- end to end through the host-buffer C-ABI (pinned host memory, copies inside)
     h_stream = torch.empty(c_bytes, dtype=torch.uint8, pin_memory=True)
@@ -411,7 +463,7 @@ def run_gpu_arm(args) -> None:
     h_out = torch.empty(n, dtype=torch.uint8, pin_memory=True)
     h_comp = torch.empty(codec.comp_capacity, dtype=torch.uint8, pin_memory=True)
     torch.cuda.synchronize(dev)
-    e2e_steps = max(1, min(args.steps, args.e2e_steps))
+    e2e_steps = args.e2e_steps or args.steps
 
     def e2e(fn):
         for _ in range(min(args.warmup, 2)):
@@ -603,13 +655,19 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--gib", type=float, default=1.0, help="corpus size per GPU in GiB")
-    ap.add_argument("--e2e-steps", type=int, default=3)
+    ap.add_argument("--e2e-steps", type=int, default=None, help="timed steps of the host-buffer legs (default: --steps)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-bst", action="store_true", help="skip the configs[3] (BST path) leg")
     ap.add_argument("--no-cli", action="store_true", help="skip the FILE* / command-line end-to-end leg")
     ap.add_argument("--no-batch64", action="store_true", help="skip the configs[4] leg (64 GiB batch, strong scaling)")
     ap.add_argument("--batch-gib", type=float, default=64.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed device legs returned in their last step as DIR/*.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or (args.e2e_steps is not None and args.e2e_steps < 1):
+        ap.error("--steps and --e2e-steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -1,5 +1,5 @@
 """Generates tests/golden/golden.json from the UNMODIFIED reference (oracle/_ref, built by
-`make -C oracle ref` from /root/reference/src).  Run in the build container only:
+`make -C oracle ref` from the reference sources, see oracle/Makefile):
 
     python tests/golden/make_golden.py
 
@@ -52,7 +52,7 @@ def main():
     varints = [{"value": v, "hex": ref.varint_encode(v).hex()}
                for v in (0, 1, 127, 128, 227, 16384, 65536, 1 << 20, 1 << 30, (1 << 31) - 1, 1 << 32, (1 << 63) + 5)]
     with open(os.path.join(HERE, "golden.json"), "w") as f:
-        json.dump({"source": "oracle/_ref built from /root/reference/src (gcc -O2)", "cases": cases,
+        json.dump({"source": "oracle/_ref built from the reference sources (gcc -O2)", "cases": cases,
                    "varints": varints}, f, indent=1)
     print(f"wrote {len(cases)} cases")
 

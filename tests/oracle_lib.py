@@ -25,7 +25,7 @@ _u8p = C.POINTER(C.c_uint8)
 
 
 def build(ref: bool = True) -> None:
-    """Compile oracle/ (and oracle/_ref when /root/reference is present)."""
+    """Compile oracle/ (and oracle/_ref when the reference sources are present: oracle/Makefile)."""
     targets = ["all"] + (["ref"] if ref else [])
     import sys
     # (make's chatter goes to stderr: bench.py's stdout is one JSON line)
@@ -107,7 +107,7 @@ class Oracle:
 
 
 class Reference:
-    """The unmodified reference, compiled from /root/reference/src by oracle/Makefile."""
+    """The unmodified reference, compiled from its own sources by oracle/Makefile (`make ref`)."""
 
     def __init__(self):
         if not os.path.exists(REF_SO):

@@ -95,7 +95,8 @@ def test_oracle_vs_reference_fuzz(oracle, reference):
             assert np.array_equal(reference.decompress(s, data.size), data), spec
 
 
-def test_reference_varint_vectors(reference, oracle):
+def test_reference_varint_vectors(oracle):
+    theirs = {v["value"]: bytes.fromhex(v["hex"]) for v in GOLDEN["varints"]}  # captured from the reference
     for v in (0, 1, 127, 128, 227, 16384, 1 << 30, (1 << 31) - 1):
-        assert reference.varint_encode(v) == oracle.varint_encode(v)
-        assert reference.varint_decode(oracle.varint_encode(v)) == v
+        assert oracle.varint_encode(v) == theirs[v]
+        assert oracle.varint_decode(theirs[v]) == (v, len(theirs[v]))
