@@ -11,8 +11,9 @@
 //     (rank = #elements before the round + popc(map up to k) - 1), then reads either the
 //     stream (literal) or the output written earlier (copy; offset < length repeats the
 //     pattern, write_copy :273-280).  A source byte produced by the very same round is
-//     followed back through the round's elements until it leaves the round or lands in a
-//     literal.
+//     resolved inside the round: k_decode_seg sends every lane to the root of its chain (a
+//     literal or a byte written earlier) by pointer doubling over shuffles, k_decode_warp follows
+//     the chain back through the round's elements.
 // Literals of 64 bytes or more are moved by the 16-byte copy loop, and the rare element kinds
 // whose header does not fit the 4 bytes a lane holds (copy-4, 4-byte literal length) take a
 // one-element path.  Copies read the output through global memory; __syncwarp() orders the
@@ -189,50 +190,123 @@ struct SegSmem {
     uint32_t bm[kRunBytes / 32 + 4]; // element starts inside the current run, one bit per output byte
 };
 
+// How produce_run resolves a copy whose source byte is produced by the same round.
+enum class Produce {
+    kShuffle, // pointer doubling over the lanes of the round (the product)
+    kFollow,  // each lane follows its chain back through the table (SNAPPY_B200_DECODE_PRODUCE=follow, A/B)
+};
+
+// Bit 31 of a source position: the byte is in the stream (relative to `in`), not in the output (relative
+// to the block's `out`, always below 65536).  A literal's stream position is below 2 * 65536 + 256.
+constexpr uint32_t kFromStream = 0x80000000u;
+
+// Table entry of an element that starts at window-relative output byte `start` (after it: `len` bytes,
+// offset `info` for a copy, stream position `info` of the first literal byte):
+//   x = start, y = offset (0: literal) | (floor(2^15/offset)+1) << 16 when the copy overlaps itself,
+//   kShuffle: z = source position of window byte 0, so that window byte k comes from position z + k (32-bit
+//             wrap-around), kFromStream set for a literal;
+//   kFollow:  (z,w) = pointer p such that window byte k is p[k] -- the stream for a literal, out + op - offset
+//             for a copy.
+// A special element (one-element path) has y = 0xffffffff and z = the stream position `pos` of its tag.
+template <Produce P>
+__device__ __forceinline__ uint4 seg_entry(const uint8_t *in, uint8_t *out, uint32_t op, uint32_t start,
+                                           const Header &h, uint32_t len, uint32_t pos, bool special)
+{
+    if (special)
+        return make_uint4(start, 0xffffffffu, pos, 0u);
+    const uint32_t off = h.is_lit ? 0u : h.info; // <= 65535 (copy-4 is special)
+    const uint32_t y = off | (off != 0 && off < len ? (32768u / off + 1u) << 16 : 0u);
+    if (P != Produce::kFollow)
+        return make_uint4(start, y, h.is_lit ? h.info - start + kFromStream : op - off, 0u);
+    const uint8_t *p = h.is_lit ? in + h.info - start : out + op - off;
+    const uint64_t pa = reinterpret_cast<uint64_t>(p);
+    return make_uint4(start, y, (uint32_t)pa, (uint32_t)(pa >> 32));
+}
+
 // Produces the output bytes [k_lo, k_hi) (window-relative) of the elements e_lo.. of the table;
 // `bm` holds their starts relative to k_lo.  Same per-byte rule as produce() above.
-__device__ __forceinline__ void produce_run(uint8_t *out, uint32_t op, uint32_t k_lo, uint32_t k_hi, uint32_t e_lo,
-                                            const SegSmem &sm, uint32_t lane)
+//
+// kShuffle: the lane of byte k = c + lane looks its element up once.  A literal, or a copy whose source
+// byte s = kk - offset lies before the round (s < c), is a root and knows the position it reads; any other
+// lane copies lane s - c < lane, its parent.  Five pointer-doubling shuffles take every lane to its root
+// (a chain inside a round has fewer than 32 links), one more fetches the root's position, and every lane
+// does exactly one load.  Rounds in which no lane has a parent skip the shuffles.  (Measured, B200, 1 GiB
+// per class: a doubling loop that ends on a ballot once every parent is a root lost on low-entropy data,
+// 3.83 against 3.64 ms; five shuffles in every round lost on text, 6.10 against 5.88 ms.)
+// Following a chain back one link computes, for k' = kk - offset, the same element look-up and kk' that
+// lane k' - c computes for itself, so both variants read the same byte.
+template <Produce P>
+__device__ __forceinline__ void produce_run(const uint8_t *__restrict__ in, uint8_t *out, uint32_t op, uint32_t k_lo,
+                                            uint32_t k_hi, uint32_t e_lo, const SegSmem &sm, uint32_t lane)
 {
     const unsigned le_mask = 0xffffffffu >> (31u - lane);
     uint32_t before = e_lo; // table index of the first element that starts in this round, if any does
     uint8_t *o = out + op + k_lo + lane;
-    for (uint32_t c = k_lo; c < k_hi; c += 32, o += 32) {
-        const unsigned B = sm.bm[(c - k_lo) >> 5];
-        uint32_t k = c + lane;
-        bool pending = k < k_hi;
-        uint32_t val = 0;
-        uint32_t r = before + __popc(B & le_mask) - 1u;
-        for (;;) {
-            if (pending) {
-                const uint4 e = sm.elems[r];
-                const uint32_t off = e.y & 0xffffu, inv = e.y >> 16;
-                uint32_t kk = k;
-                if (inv) { // write_copy :273-280: byte i comes from i mod offset when the copy overlaps itself
-                    const uint32_t i = k - e.x;
-                    kk = e.x + i - off * ((i * inv) >> 15);
-                }
-                if (off == 0 || kk < c + off) {
-                    // a literal, or a copy whose source was written by an earlier step / round
-                    const uint8_t *p = reinterpret_cast<const uint8_t *>(((uint64_t)e.w << 32) | e.z);
-                    val = p[kk];
-                    pending = false;
-                } else {
-                    k = kk - off; // produced by this very round: follow it back
-                    r = before + __popc(B & (0xffffffffu >> (31u - (k - c)))) - 1u;
-                }
+    if constexpr (P != Produce::kFollow) {
+        for (uint32_t c = k_lo; c < k_hi; c += 32, o += 32) {
+            const unsigned B = sm.bm[(c - k_lo) >> 5];
+            // every lane's look-up is a valid table entry (the element at or before it), also past k_hi
+            const uint4 e = sm.elems[before + __popc(B & le_mask) - 1u];
+            const uint32_t off = e.y & 0xffffu, inv = e.y >> 16;
+            uint32_t kk = c + lane;
+            if (inv) { // write_copy :273-280: byte i comes from i mod offset when the copy overlaps itself
+                const uint32_t i = kk - e.x;
+                kk = e.x + i - off * ((i * inv) >> 15);
             }
-            if (!__any_sync(kFull, pending))
-                break;
+            uint32_t src = e.z + kk;
+            // produced by this very round: the parent is a lower lane (a lane past k_hi has no children)
+            uint32_t parent = off != 0 && kk >= c + off ? kk - off - c : lane;
+            if (__any_sync(kFull, parent != lane)) {
+#pragma unroll
+                for (int d = 0; d < 5; ++d)
+                    parent = __shfl_sync(kFull, parent, parent);
+                src = __shfl_sync(kFull, src, parent);
+            }
+            if (c + lane < k_hi) {
+                const uint8_t *base = (src & kFromStream) ? in : out;
+                *o = base[src & ~kFromStream];
+            }
+            before += __popc(B);
+            __syncwarp(); // the next round may read what this one wrote
         }
-        if (c + lane < k_hi)
-            *o = (uint8_t)val;
-        before += __popc(B);
-        __syncwarp(); // the next round may read what this one wrote
+    } else {
+        for (uint32_t c = k_lo; c < k_hi; c += 32, o += 32) {
+            const unsigned B = sm.bm[(c - k_lo) >> 5];
+            uint32_t k = c + lane;
+            bool pending = k < k_hi;
+            uint32_t val = 0;
+            uint32_t r = before + __popc(B & le_mask) - 1u;
+            for (;;) {
+                if (pending) {
+                    const uint4 e = sm.elems[r];
+                    const uint32_t off = e.y & 0xffffu, inv = e.y >> 16;
+                    uint32_t kk = k;
+                    if (inv) { // write_copy :273-280: byte i comes from i mod offset when the copy overlaps itself
+                        const uint32_t i = k - e.x;
+                        kk = e.x + i - off * ((i * inv) >> 15);
+                    }
+                    if (off == 0 || kk < c + off) {
+                        // a literal, or a copy whose source was written by an earlier step / round
+                        const uint8_t *p = reinterpret_cast<const uint8_t *>(((uint64_t)e.w << 32) | e.z);
+                        val = p[kk];
+                        pending = false;
+                    } else {
+                        k = kk - off; // produced by this very round: follow it back
+                        r = before + __popc(B & (0xffffffffu >> (31u - (k - c)))) - 1u;
+                    }
+                }
+                if (!__any_sync(kFull, pending))
+                    break;
+            }
+            if (c + lane < k_hi)
+                *o = (uint8_t)val;
+            before += __popc(B);
+            __syncwarp(); // the next round may read what this one wrote
+        }
     }
 }
 
-template <int MINB>
+template <int MINB, Produce P>
 __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restrict__ stream, uint64_t body_offset,
                                                          const uint64_t *__restrict__ offsets,
                                                          const uint4 *__restrict__ starts, uint64_t total_out,
@@ -272,26 +346,28 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
     uint8_t *out = out_base + blk * (uint64_t)kBlock;
     const uint64_t oleft = total_out - blk * (uint64_t)kBlock;
     const uint32_t olen = oleft < kBlock ? (uint32_t)oleft : kBlock;
+    const uint4 *__restrict__ seg_starts = starts + t0;
+    const uint32_t ns = (uint32_t)(t1 - t0); // segments t0..t1 are s = 0..ns
     const uint32_t w = lane >> 3, sh = (lane & 7u) * 4u; // my nibble of the 128-bit start map
     for (uint32_t i = lane; i < 256; i += 32)
         sm.lut[i] = (uint16_t)tag_facts(i);
     __syncwarp();
 
     uint32_t op = 0, err = 0;
-    for (uint64_t t = t0; t <= t1 && !err; ++t) {
-        const uint4 sv = __ldg(starts + t);
+    for (uint32_t s = 0; s <= ns && !err; ++s) {
+        const uint4 sv = __ldg(seg_starts + s);
         uint32_t R[4] = {sv.x, sv.y, sv.z, sv.w};
-        const uint32_t seg_lo = (uint32_t)((t - t0) * kSegBytes);
+        const uint32_t seg_lo = s * kSegBytes;
         // the block is one serial chain: have the stream (and its maps) on their way before they are needed
         // (every 8 segments: the 8 stream lines 16..23 segments ahead, one lane each, and the line of their maps)
-        if (((t - t0) & 7u) == 0 && lane <= 8 && t + 16 + lane <= t1) {
+        if ((s & 7u) == 0 && lane <= 8 && s + 16 + lane <= ns) {
             if (lane < 8)
                 prefetch_l2(in + seg_lo + (16 + lane) * kSegBytes);
             else
-                prefetch_l2(starts + t + 16);
+                prefetch_l2(seg_starts + s + 16);
         }
         // keep only the starts that belong to this block (only the first / last segment can hold others)
-        if (t == t0 || t == t1)
+        if (s == 0 || s == ns)
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 const uint32_t lo = seg_lo + 32 * q; // stream position of bit 0 of this word
@@ -354,34 +430,10 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
         const uint32_t T = T64;
         const unsigned S = __ballot_sync(kFull, sp0 || sp1);
         // ---- the table
-        if (has0) {
-            uint32_t y = 0;
-            const uint8_t *p = in + h0.info - start0; // literal: byte k of the window = stream byte info + (k - start)
-            if (sp0) {
-                y = 0xffffffffu; // not for produce_run: z = stream position of the tag
-                p = reinterpret_cast<const uint8_t *>((uintptr_t)pos0);
-            } else if (!h0.is_lit) {
-                const uint32_t off = h0.info; // <= 65535 (copy-4 is special)
-                y = off | (off < len0 ? (32768u / off + 1u) << 16 : 0u);
-                p = out + op - off; // byte k of the window = output byte op + k - off
-            }
-            const uint64_t pa = reinterpret_cast<uint64_t>(p);
-            sm.elems[rank] = make_uint4(start0, y, (uint32_t)pa, (uint32_t)(pa >> 32));
-        }
-        if (has1) {
-            uint32_t y = 0;
-            const uint8_t *p = in + h1.info - start1;
-            if (sp1) {
-                y = 0xffffffffu;
-                p = reinterpret_cast<const uint8_t *>((uintptr_t)pos1);
-            } else if (!h1.is_lit) {
-                const uint32_t off = h1.info;
-                y = off | (off < len1 ? (32768u / off + 1u) << 16 : 0u);
-                p = out + op - off;
-            }
-            const uint64_t pa = reinterpret_cast<uint64_t>(p);
-            sm.elems[rank + 1] = make_uint4(start1, y, (uint32_t)pa, (uint32_t)(pa >> 32));
-        }
+        if (has0)
+            sm.elems[rank] = seg_entry<P>(in, out, op, start0, h0, len0, pos0, sp0);
+        if (has1)
+            sm.elems[rank + 1] = seg_entry<P>(in, out, op, start1, h1, len1, pos1, sp1);
         if (S == 0) {
             // ---- the ordinary segment: one run
             const uint32_t words = (T + 31) >> 5;
@@ -393,7 +445,7 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
             if (has1)
                 atomicOr(&sm.bm[start1 >> 5], 1u << (start1 & 31u));
             __syncwarp(); // also: stores of earlier steps are visible to every lane from here
-            produce_run(out, op, 0, T, 0, sm, lane);
+            produce_run<P>(in, out, op, 0, T, 0, sm, lane);
         } else {
             // ---- runs of ordinary elements between the special ones (long literals, copy-4, ...)
             __syncwarp();
@@ -419,7 +471,7 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
                     if (has1 && rank + 1 >= e_lo && rank + 1 < e_hi)
                         atomicOr(&sm.bm[(start1 - k_lo) >> 5], 1u << ((start1 - k_lo) & 31u));
                     __syncwarp();
-                    produce_run(out, op, k_lo, k_hi, e_lo, sm, lane);
+                    produce_run<P>(in, out, op, k_lo, k_hi, e_lo, sm, lane);
                 }
                 if (e_hi < ne) {
                     uint32_t ip = sm.elems[e_hi].z, o2 = op + k_hi;
@@ -651,7 +703,7 @@ cudaError_t launch_copy_literal_blocks(const uint8_t *, uint64_t, const uint64_t
 // above (k_decode_seg) preceded by k_copy_literal_blocks, which moves the blocks that are a single literal
 // (incompressible data) with plain 16-byte vector copies; inputs of at most 32 blocks go to the tile decoder
 // (k_decode_tile), whose eight warps per block give the lower latency.  Three other designs were built and measured in
-// round 2 and lost (1 GiB mixed corpus: seg 4.1 ms; profiles/r02_*): SNAPPY_B200_DECODER=tile selects the
+// round 2 and lost (1 GiB mixed corpus: seg 3.6 ms in round 2, 3.36 ms in round 3; profiles/r02_*): SNAPPY_B200_DECODER=tile selects the
 // one-CTA-per-block decoder with the whole 64 KiB block in shared memory (decode_tile.cu, 32 ms), =win the
 // sub-warp-group-per-block decoder with a sliding shared-memory window (decode_win.cu, 9.3 ms), =lane the
 // one-lane-per-block sequential decoder (decode_lane.cu, 18.7 ms; 9.4 ms/GiB at 4 GiB).  All four are
@@ -700,8 +752,17 @@ cudaError_t launch_decode_seg(const uint8_t *d_stream, uint64_t body_offset, con
     }
     // two blocks (warps) per CTA and a 48-register cap: 40 warps per SM instead of the 32 that one-warp
     // CTAs allow (measured: 64 registers / 32 warps 6.92, 48 / 40 6.72, 40 / 48 6.84 ms per GiB, K0 included)
-    k_decode_seg<20><<<(unsigned)((n_blocks + 1) / 2), 64, 0, st>>>(d_stream, body_offset, d_offsets, d_starts, total_out,
-                                                                    d_out, d_status, n_blocks, blk_base, d_order);
+    static const char produce = [] { // A/B: SNAPPY_B200_DECODE_PRODUCE=follow selects the follow-back loop
+        const char *v = getenv("SNAPPY_B200_DECODE_PRODUCE");
+        return v ? v[0] : 's';
+    }();
+    const unsigned grid = (unsigned)((n_blocks + 1) / 2);
+    if (produce == 'f')
+        k_decode_seg<20, Produce::kFollow><<<grid, 64, 0, st>>>(d_stream, body_offset, d_offsets, d_starts, total_out,
+                                                                d_out, d_status, n_blocks, blk_base, d_order);
+    else
+        k_decode_seg<20, Produce::kShuffle><<<grid, 64, 0, st>>>(d_stream, body_offset, d_offsets, d_starts, total_out,
+                                                                 d_out, d_status, n_blocks, blk_base, d_order);
     *launches += 1;
     return cudaGetLastError();
 }
