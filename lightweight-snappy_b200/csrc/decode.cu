@@ -659,6 +659,31 @@ cudaError_t launch_decode(const uint8_t *d_stream, const uint64_t *d_offsets, ui
     return cudaGetLastError();
 }
 
+namespace {
+
+// Runs in front of k_decode_seg: a block that is one literal (incompressible data) is moved stream -> output by the
+// whole CTA with 16-byte vector copies, and k_decode_seg skips it.
+__global__ void __launch_bounds__(256) k_copy_literal_blocks(const uint8_t *__restrict__ stream, uint64_t body_offset,
+                                                             const uint64_t *__restrict__ offsets, uint64_t total_out,
+                                                             uint8_t *out_base, const uint32_t *__restrict__ status,
+                                                             uint64_t n_blocks)
+{
+    const uint64_t blk = blockIdx.x;
+    if (*reinterpret_cast<const volatile uint32_t *>(status) != 0)
+        return;
+    const uint64_t c0 = offsets[blk], c1 = offsets[blk + 1];
+    if (c1 <= c0 || c0 < body_offset || c1 > offsets[n_blocks] || c1 - c0 > 2u * kBlock)
+        return; // k_decode_seg reports it
+    const uint64_t oleft = total_out - blk * (uint64_t)kBlock;
+    const uint32_t olen = oleft < kBlock ? (uint32_t)oleft : kBlock;
+    if (!one_literal_block(stream, c0, c1, olen))
+        return;
+    const uint32_t hdr = ((uint32_t)__ldg(stream + c0) >> 2) - 58u; // tag + length bytes
+    coop_copy_ro(out_base + blk * (uint64_t)kBlock, stream + c0 + hdr, olen, threadIdx.x, 256);
+}
+
+} // namespace
+
 // A block is one serial chain (about 2 ms for a text block, 1.5 ms for a low-entropy one, nothing for a block
 // that k_copy_literal_blocks has moved), and 1 GiB is fewer than two waves of them: started in stream order the
 // last wave ends with a few long blocks on an otherwise idle GPU.  The blocks are therefore handed out longest
@@ -690,24 +715,12 @@ __global__ void __launch_bounds__(1024) k_block_order(const uint64_t *__restrict
 cudaError_t launch_decode_tile(const uint8_t *, uint64_t, const uint64_t *, const uint4 *, const uint64_t *, uint64_t,
                                uint64_t, uint8_t *, uint32_t *, uint64_t, cudaStream_t, uint64_t *); // decode_tile.cu
 
-cudaError_t launch_decode_win(const uint8_t *, uint64_t, const uint64_t *, const uint4 *, uint64_t, uint64_t, uint8_t *,
-                              uint32_t *, uint64_t, cudaStream_t, uint64_t *); // decode_win.cu
-
-cudaError_t launch_decode_lane(const uint8_t *, uint64_t, const uint64_t *, uint64_t, uint64_t, uint8_t *, uint32_t *,
-                               uint64_t, bool, cudaStream_t, uint64_t *); // decode_lane.cu
-
-cudaError_t launch_copy_literal_blocks(const uint8_t *, uint64_t, const uint64_t *, uint64_t, uint64_t, uint8_t *,
-                                       const uint32_t *, cudaStream_t, uint64_t *); // decode_lane.cu
-
-// Decoder for the maps K0 leaves behind.  The product path is the warp-per-block, segment-driven decoder
-// above (k_decode_seg) preceded by k_copy_literal_blocks, which moves the blocks that are a single literal
-// (incompressible data) with plain 16-byte vector copies; inputs of at most 32 blocks go to the tile decoder
-// (k_decode_tile), whose eight warps per block give the lower latency.  Three other designs were built and measured in
-// round 2 and lost (1 GiB mixed corpus: seg 3.6 ms in round 2, 3.36 ms in round 3; profiles/r02_*): SNAPPY_B200_DECODER=tile selects the
-// one-CTA-per-block decoder with the whole 64 KiB block in shared memory (decode_tile.cu, 32 ms), =win the
-// sub-warp-group-per-block decoder with a sliding shared-memory window (decode_win.cu, 9.3 ms), =lane the
-// one-lane-per-block sequential decoder (decode_lane.cu, 18.7 ms; 9.4 ms/GiB at 4 GiB).  All four are
-// bit-exact (tests/test_gpu_parity.py::test_alternative_decoders).
+// Decoder for the maps K0 leaves behind.  Inputs of at most 32 blocks go to the tile decoder (k_decode_tile), whose
+// eight warps per block give the lower latency; larger ones to the warp-per-block, segment-driven decoder above
+// (k_decode_seg), preceded by k_copy_literal_blocks, which moves the blocks that are a single literal.
+// SNAPPY_B200_DECODER=seg|tile (read once per process) forces one of the two on any input, so that both can be tested
+// on either side of the threshold; unset or =auto picks by size.  The other block decoders that were built and
+// measured, and why they lost, are in DESIGN.md §4.
 cudaError_t launch_decode_seg(const uint8_t *d_stream, uint64_t body_offset, const uint64_t *d_offsets,
                               const uint4 *d_starts, const uint64_t *d_outoff, uint64_t n_blocks, uint64_t total_out,
                               uint8_t *d_out, uint32_t *d_status, uint64_t blk_base, cudaStream_t st,
@@ -727,18 +740,14 @@ cudaError_t launch_decode_seg(const uint8_t *d_stream, uint64_t body_offset, con
     // API, 64 KiB: 1.18 -> 0.72 ms; 1 MiB: 1.40 -> 0.88 ms; 16 MiB: 2.78 vs 3.70 ms the other way round).
     constexpr uint64_t kTileMaxBlocks = 32;
     const char which = which_env != 'a' ? which_env : (n_blocks <= kTileMaxBlocks && d_outoff ? 't' : 's');
-    if (which == 'l')
-        return launch_decode_lane(d_stream, body_offset, d_offsets, n_blocks, total_out, d_out, d_status, blk_base, true,
-                                  st, launches);
     if (which == 't')
         return launch_decode_tile(d_stream, body_offset, d_offsets, d_starts, d_outoff, n_blocks, total_out, d_out,
                                   d_status, blk_base, st, launches);
 
-    if (which == 'w')
-        return launch_decode_win(d_stream, body_offset, d_offsets, d_starts, n_blocks, total_out, d_out, d_status,
-                                 blk_base, st, launches);
-    cudaError_t e = launch_copy_literal_blocks(d_stream, body_offset, d_offsets, n_blocks, total_out, d_out, d_status, st,
-                                               launches);
+    k_copy_literal_blocks<<<(unsigned)n_blocks, 256, 0, st>>>(d_stream, body_offset, d_offsets, total_out, d_out, d_status,
+                                                             n_blocks);
+    *launches += 1;
+    cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess)
         return e;
     // The order array lives in the memory of K0's per-segment output offsets, which this decoder does not need

@@ -1,7 +1,8 @@
 // lanecopy.cuh -- byte moves done by ONE lane, any alignment, 16 bytes per step with word accesses.
 //
-// The decoders give every element (literal or copy, src/snappy_decompression.c:232-239, :273-280) to one
-// lane; the destination is always shared memory, the source shared or global memory (generic pointers).
+// The tile decoder (decode_tile.cu) gives every element (literal or copy, src/snappy_decompression.c:232-239,
+// :273-280) to one lane; the destination is always shared memory, the source shared or global memory (generic
+// pointers).
 #pragma once
 
 #include "common.cuh"
