@@ -92,7 +92,8 @@ int snappy_b200_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode,
                                 uint32_t *d_status, void *d_workspace, size_t workspace_bytes, void *stream);
 
 /* Decodes n_blocks blocks whose stream offsets are given (d_block_offsets[n_blocks+1]);
- * block i produces bytes [i*65536, min(total_out, (i+1)*65536)) of d_out.  *d_status is
+ * block i produces bytes [i*65536, min(total_out, (i+1)*65536)) of d_out.  Valid raw Snappy the block
+ * decoder does not take (see snappy_b200_decompress_host_indexed) gives SNAPPY_B200_ST_FRAMING.  *d_status is
  * OR-ed into, not reset: the caller zeroes it, and a non-zero status on entry (e.g. left by
  * a failed snappy_b200_index_device on the same stream) turns the call into a no-op.     */
 int snappy_b200_decompress_device_indexed(const uint8_t *d_stream, const uint64_t *d_block_offsets,
@@ -151,8 +152,12 @@ int snappy_b200_decompress_host(const void *stream, uint64_t stream_bytes, void 
  * stream offset at which the b-th 64 KiB block starts, block_offsets[snappy_b200_block_count(n)]
  * the stream length.  The stream itself is unchanged (byte-identical to the reference); a decoder
  * that is handed the index does not have to discover the block boundaries (no K0).  The
- * indexed decoder checks the index against the stream and reports SNAPPY_B200_ERR_CORRUPT /
- * _FRAMING when they disagree.                                                            */
+ * indexed decoder checks the index against the stream and reports SNAPPY_B200_ERR_CORRUPT when
+ * they disagree.  Valid raw Snappy that the block decoders do not take -- elements that straddle
+ * a block, copies into an earlier block, blocks longer than 2 * 65536 stream bytes (non-minimal
+ * encodings) -- is decoded by the general decoder, as snappy_b200_decompress_host does.  A stream
+ * may be up to 6 bytes per output byte long (1-byte literals with a 4-byte length) plus the
+ * varint; only a longer one is rejected before it is decoded.                              */
 int snappy_b200_compress_host_indexed(const void *in, uint64_t n_bytes, int mode, void *out, uint64_t out_capacity,
                                       uint64_t *out_bytes, uint64_t *block_offsets);
 int snappy_b200_decompress_host_indexed(const void *stream, uint64_t stream_bytes, const uint64_t *block_offsets,
@@ -171,8 +176,9 @@ int snappy_b200_compress_host_multi_range(const void *in, uint64_t n_bytes, int 
  * one worker thread and one arena per device, no collective and no peer copy -- the only cross-device datum
  * is the compressed size of every partition (an exclusive scan on the host places the partitions).  The
  * stream is byte-identical to the one-device stream.  The index-less decode first runs K0 over the whole
- * stream on the current device.  The plain calls above forward here when SNAPPY_B200_DEVICES=N (N > 1) is set
- * and the data is at least 64 MiB.                                                                      */
+ * stream on the current device.  The plain calls above forward here when SNAPPY_B200_DEVICES=N (N > 1) is set,
+ * more than one device is present and the data is at least 64 MiB.  Streams the block decoders do not take go
+ * to the general decoder on the current device, as in the one-device calls.                               */
 int snappy_b200_compress_host_multi(const void *in, uint64_t n_bytes, int mode, void *out, uint64_t out_capacity,
                                     uint64_t *out_bytes, uint64_t *block_offsets, int n_devices);
 int snappy_b200_decompress_host_multi(const void *stream, uint64_t stream_bytes, void *out, uint64_t out_capacity,

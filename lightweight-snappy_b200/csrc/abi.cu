@@ -303,7 +303,8 @@ int snappy_b200_decompress_device_async(const uint8_t *d_stream, uint64_t stream
     if (workspace_bytes < snappy_b200_decompress_async_workspace_bytes(stream_bytes, total_out))
         return fail(SNAPPY_B200_ERR_ARG, "workspace too small (see snappy_b200_decompress_async_workspace_bytes)");
     if (total_out == 0)
-        return SNAPPY_B200_OK;
+        return stream_bytes == body_offset ? SNAPPY_B200_OK
+                                           : fail(SNAPPY_B200_ERR_CORRUPT, "trailing bytes after an empty stream");
     const uint64_t nb = (total_out + kBlock - 1) / kBlock;
     uint64_t *offs = d_block_offsets
                          ? d_block_offsets

@@ -326,8 +326,11 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
     const uint64_t c0 = offsets[blk], c1 = offsets[blk + 1];
     const uint64_t stream_bytes = offsets[n_blocks];
     if (c1 <= c0 || c0 < body_offset || c1 > stream_bytes || c1 - c0 > 2u * kBlock) {
+        // a range that does not fit the stream is an error; a block of more than 2 * 65536 stream bytes is valid
+        // raw Snappy (non-minimal encodings) that only the general decoder takes
         if (lane == 0)
-            atomicOr(status, SNAPPY_B200_ST_CORRUPT);
+            atomicOr(status, c1 > c0 && c0 >= body_offset && c1 <= stream_bytes ? SNAPPY_B200_ST_FRAMING
+                                                                                 : SNAPPY_B200_ST_CORRUPT);
         return;
     }
     {
@@ -502,9 +505,10 @@ __global__ void __launch_bounds__(32) k_decode_warp(const uint8_t *__restrict__ 
     const uint64_t c0 = offsets[blk], c1 = offsets[blk + 1];
     const uint64_t stream_bytes = offsets[gridDim.x]; // entry n_blocks of the index = end of the stream
     const uint64_t clen64 = c1 - c0;
-    if (c1 < c0 || c1 > stream_bytes || clen64 > 2u * kBlock) { // a block never needs more than 65536+1010
+    if (c1 < c0 || c1 > stream_bytes || clen64 > 2u * kBlock) { // a compressor's block never needs more than 65536+1010
+        // a longer block is valid raw Snappy (non-minimal encodings) that only the general decoder takes
         if (lane == 0)
-            atomicOr(status, SNAPPY_B200_ST_CORRUPT);
+            atomicOr(status, c1 < c0 || c1 > stream_bytes ? SNAPPY_B200_ST_CORRUPT : SNAPPY_B200_ST_FRAMING);
         return;
     }
     const uint8_t *__restrict__ in = stream + c0;
@@ -673,7 +677,7 @@ __global__ void __launch_bounds__(256) k_copy_literal_blocks(const uint8_t *__re
         return;
     const uint64_t c0 = offsets[blk], c1 = offsets[blk + 1];
     if (c1 <= c0 || c0 < body_offset || c1 > offsets[n_blocks] || c1 - c0 > 2u * kBlock)
-        return; // k_decode_seg reports it
+        return; // k_decode_seg reports it (a bad range as ST_CORRUPT, an oversized block as ST_FRAMING)
     const uint64_t oleft = total_out - blk * (uint64_t)kBlock;
     const uint32_t olen = oleft < kBlock ? (uint32_t)oleft : kBlock;
     if (!one_literal_block(stream, c0, c1, olen))

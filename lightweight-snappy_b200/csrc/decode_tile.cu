@@ -165,8 +165,11 @@ __global__ void __launch_bounds__(kThreads, 3)
     const uint64_t c0 = offsets[blk], c1 = offsets[blk + 1];
     const uint64_t stream_bytes = offsets[n_blocks];
     if (c1 <= c0 || c0 < body_offset || c1 > stream_bytes || c1 - c0 > 2u * kBlock) {
+        // a range that does not fit the stream is an error; a block of more than 2 * 65536 stream bytes is valid
+        // raw Snappy (non-minimal encodings) that only the general decoder takes
         if (tid == 0)
-            atomicOr(status, SNAPPY_B200_ST_CORRUPT);
+            atomicOr(status, c1 > c0 && c0 >= body_offset && c1 <= stream_bytes ? SNAPPY_B200_ST_FRAMING
+                                                                                 : SNAPPY_B200_ST_CORRUPT);
         return;
     }
     uint8_t *out = out_base + blk * (uint64_t)kBlock;
@@ -385,7 +388,10 @@ __global__ void __launch_bounds__(kThreads, 3)
         }
         __syncthreads();
     }
-    if (tid == 0 && sm.produced != olen)
+    // a refused element has produced nothing: the byte count is only a finding when every element was taken
+    // (a valid unframed stream must report ST_FRAMING alone, so that the general decoder takes it)
+    const int refused = __syncthreads_or(err != 0);
+    if (tid == 0 && !refused && sm.produced != olen)
         err |= SNAPPY_B200_ST_CORRUPT;
     if (err)
         atomicOr(status, err);

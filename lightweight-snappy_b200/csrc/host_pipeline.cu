@@ -32,6 +32,7 @@
 #include "common.cuh"
 
 namespace sb200 {
+int decompress_host_general(const void *stream, uint64_t stream_bytes, void *out, uint64_t *out_bytes);
 int fail_msg(int code, const char *msg);
 void clear_error();
 int cuda_fail_msg(cudaError_t e, const char *what);
@@ -74,6 +75,14 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 inline uint64_t max_compressed(uint64_t n)
 {
     return n ? 10 + n + ((n + kBlock - 1) / kBlock) * 1010 : 0;
+}
+
+// The longest valid encoding of `total` output bytes: one 1-byte literal with a 4-byte length (6 stream bytes)
+// per output byte.  Streams between max_compressed(total) and this are valid raw Snappy that no compressor
+// emits; they are decoded (by the general decoder when their blocks are too long for the block decoders).
+inline bool longer_than_any_encoding(uint64_t stream_bytes, uint64_t hdr, uint64_t total)
+{
+    return (stream_bytes - hdr + 5) / 6 > total;
 }
 
 unsigned host_varint_decode(const uint8_t *p, uint64_t avail, uint64_t *out)
@@ -201,6 +210,21 @@ int env_devices()
     const char *v = getenv("SNAPPY_B200_DEVICES");
     const int n = v ? atoi(v) : 1;
     return n < 1 ? 1 : n;
+}
+// Devices a decompress call would shard over: SNAPPY_B200_DEVICES, at most the devices present.  The decode
+// forwards to the multi-device calls only when this is above 1: with a single device those calls come back
+// to the one-device path.
+int decode_devices()
+{
+    const int want = env_devices();
+    int n = 0;
+    if (want < 2)
+        return 1;
+    if (cudaGetDeviceCount(&n) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return 1;
+    }
+    return std::min(want, n);
 }
 constexpr uint64_t kMultiMin = 64ull << 20;
 
@@ -554,10 +578,10 @@ static int decompress_host_framed(const void *stream, uint64_t stream_bytes, voi
                                    : fail_msg(SNAPPY_B200_ERR_CORRUPT, "trailing bytes after an empty stream");
     if (!out)
         return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
-    if (stream_bytes > max_compressed(total) + 16)
+    if (longer_than_any_encoding(stream_bytes, hdr, total))
         return fail_msg(SNAPPY_B200_ERR_CORRUPT, "stream is longer than any encoding of its declared length");
-    if (env_devices() > 1 && total >= kMultiMin)
-        return snappy_b200_decompress_host_multi(stream, stream_bytes, out, out_capacity, out_bytes, env_devices());
+    if (decode_devices() > 1 && total >= kMultiMin)
+        return snappy_b200_decompress_host_multi(stream, stream_bytes, out, out_capacity, out_bytes, decode_devices());
 
     std::lock_guard<std::mutex> lock(g_ctx.mu);
     CU(g_ctx.init(), "context init");
@@ -646,9 +670,13 @@ static int decompress_host_framed(const void *stream, uint64_t stream_bytes, voi
     return SNAPPY_B200_OK;
 }
 
-// Valid raw Snappy that is not framed in 64 KiB blocks (straddling elements, copies into earlier blocks):
-// decoded like the reference does, one element after the other (k_decode_sequential).
-static int decompress_host_general(const void *stream, uint64_t stream_bytes, void *out, uint64_t *out_bytes)
+} // extern "C"
+
+namespace sb200 {
+// Valid raw Snappy that is not framed in 64 KiB blocks (straddling elements, copies into earlier blocks, blocks
+// longer than the block decoders take): decoded like the reference does, one element after the other
+// (k_decode_sequential).  The caller has checked the arguments and that the output fits.
+int decompress_host_general(const void *stream, uint64_t stream_bytes, void *out, uint64_t *out_bytes)
 {
     HostCtx &g_ctx = current_ctx();
     uint64_t total = 0;
@@ -675,6 +703,9 @@ static int decompress_host_general(const void *stream, uint64_t stream_bytes, vo
     *out_bytes = total;
     return SNAPPY_B200_OK;
 }
+} // namespace sb200
+
+extern "C" {
 
 int snappy_b200_decompress_host(const void *stream, uint64_t stream_bytes, void *out, uint64_t out_capacity,
                                 uint64_t *out_bytes)
@@ -719,7 +750,7 @@ int snappy_b200_decompress_file(FILE *in, FILE *out)
         return fail_msg(SNAPPY_B200_ERR_CORRUPT, "bad varint preamble");
     if (total == 0)
         return L == hdr ? SNAPPY_B200_OK : fail_msg(SNAPPY_B200_ERR_CORRUPT, "trailing bytes after an empty stream");
-    if (L > max_compressed(total) + 16)
+    if (longer_than_any_encoding(L, hdr, total))
         return fail_msg(SNAPPY_B200_ERR_CORRUPT, "stream is longer than any encoding of its declared length");
     if (total >= (1ull << 40))
         return 1;
@@ -804,8 +835,8 @@ int snappy_b200_decompress_file(FILE *in, FILE *out)
 // ---- decode with the side index: no K0.  The stream goes up in pieces cut at block boundaries
 // (growing like the index-less path's), every piece is decoded by the window decoder as soon as it
 // has landed and downloaded while the next one is in flight.
-int snappy_b200_decompress_host_indexed(const void *stream, uint64_t stream_bytes, const uint64_t *block_offsets,
-                                        uint64_t n_blocks, void *out, uint64_t out_capacity, uint64_t *out_bytes)
+static int decompress_host_indexed_blocks(const void *stream, uint64_t stream_bytes, const uint64_t *block_offsets,
+                                          uint64_t n_blocks, void *out, uint64_t out_capacity, uint64_t *out_bytes)
 {
     clear_error();
     HostCtx &g_ctx = current_ctx();
@@ -830,11 +861,14 @@ int snappy_b200_decompress_host_indexed(const void *stream, uint64_t stream_byte
     if (block_offsets[0] != hdr || block_offsets[n_blocks] != stream_bytes)
         return fail_msg(SNAPPY_B200_ERR_CORRUPT, "the index does not span the stream");
     for (uint64_t b = 0; b < n_blocks; ++b)
-        if (block_offsets[b + 1] <= block_offsets[b] || block_offsets[b + 1] - block_offsets[b] > 2u * kBlock)
-            return fail_msg(SNAPPY_B200_ERR_CORRUPT, "the index is not increasing / a block is larger than any 64 KiB block can be");
-    if (env_devices() > 1 && total >= kMultiMin)
+        if (block_offsets[b + 1] <= block_offsets[b])
+            return fail_msg(SNAPPY_B200_ERR_CORRUPT, "the index is not increasing");
+    for (uint64_t b = 0; b < n_blocks; ++b)
+        if (block_offsets[b + 1] - block_offsets[b] > 2u * kBlock)
+            return fail_msg(SNAPPY_B200_ERR_FRAMING, "a block is longer than the block decoders take (2 * 65536 stream bytes)");
+    if (decode_devices() > 1 && total >= kMultiMin)
         return snappy_b200_decompress_host_indexed_multi(stream, stream_bytes, block_offsets, n_blocks, out, out_capacity,
-                                                         out_bytes, env_devices());
+                                                         out_bytes, decode_devices());
 
     std::lock_guard<std::mutex> lock(g_ctx.mu);
     CU(g_ctx.init(), "context init");
@@ -885,6 +919,17 @@ int snappy_b200_decompress_host_indexed(const void *stream, uint64_t stream_byte
     return SNAPPY_B200_OK;
 }
 
+int snappy_b200_decompress_host_indexed(const void *stream, uint64_t stream_bytes, const uint64_t *block_offsets,
+                                        uint64_t n_blocks, void *out, uint64_t out_capacity, uint64_t *out_bytes)
+{
+    const int rc = decompress_host_indexed_blocks(stream, stream_bytes, block_offsets, n_blocks, out, out_capacity,
+                                                  out_bytes);
+    if (rc != SNAPPY_B200_ERR_FRAMING)
+        return rc;
+    clear_error();
+    return decompress_host_general(stream, stream_bytes, out, out_bytes); // (all arguments were checked above)
+}
+
 // ---- device-level index-less decode (include/snappy_b200.h): the same piecewise loop on a
 // device-resident stream, with a library-owned second stream for the decode kernels.
 // A device-resident stream is decoded as ONE piece: K0 has about 2 ms of latency-bound fixed cost
@@ -924,7 +969,8 @@ int snappy_b200_decompress_device(const uint8_t *d_stream, uint64_t stream_bytes
     if (workspace_bytes < snappy_b200_decompress_workspace_bytes(stream_bytes, total_out))
         return fail_msg(SNAPPY_B200_ERR_ARG, "workspace too small (see snappy_b200_decompress_workspace_bytes)");
     if (total_out == 0)
-        return SNAPPY_B200_OK;
+        return stream_bytes == body_offset ? SNAPPY_B200_OK
+                                           : fail_msg(SNAPPY_B200_ERR_CORRUPT, "trailing bytes after an empty stream");
     std::lock_guard<std::mutex> lock(g_ctx.mu);
     CU(g_ctx.init(), "context init");
     const uint64_t piece = device_piece_bytes(stream_bytes);

@@ -19,6 +19,7 @@
 #include "common.cuh"
 
 namespace sb200 {
+int decompress_host_general(const void *stream, uint64_t stream_bytes, void *out, uint64_t *out_bytes);
 int fail_msg(int code, const char *msg);
 int cuda_fail_msg(cudaError_t e, const char *what);
 int status_error(uint32_t st);
@@ -255,9 +256,9 @@ int snappy_b200_compress_host_multi_range(const void *in, uint64_t n_bytes, int 
     return SNAPPY_B200_OK;
 }
 
-int snappy_b200_decompress_host_indexed_multi(const void *stream, uint64_t stream_bytes, const uint64_t *block_offsets,
-                                              uint64_t n_blocks, void *out, uint64_t out_capacity, uint64_t *out_bytes,
-                                              int n_devices)
+static int decompress_host_indexed_multi_blocks(const void *stream, uint64_t stream_bytes, const uint64_t *block_offsets,
+                                                uint64_t n_blocks, void *out, uint64_t out_capacity, uint64_t *out_bytes,
+                                                int n_devices)
 {
     clear_error();
     if (!out_bytes || (stream_bytes && !stream) || !block_offsets)
@@ -293,9 +294,11 @@ int snappy_b200_decompress_host_indexed_multi(const void *stream, uint64_t strea
     if (block_offsets[0] != hdr || block_offsets[n_blocks] != stream_bytes)
         return fail_msg(SNAPPY_B200_ERR_CORRUPT, "the index does not span the stream");
     for (uint64_t b = 0; b < n_blocks; ++b)
-        if (block_offsets[b + 1] <= block_offsets[b] || block_offsets[b + 1] - block_offsets[b] > 2u * kBlock)
-            return fail_msg(SNAPPY_B200_ERR_CORRUPT,
-                            "the index is not increasing / a block is larger than any 64 KiB block can be");
+        if (block_offsets[b + 1] <= block_offsets[b])
+            return fail_msg(SNAPPY_B200_ERR_CORRUPT, "the index is not increasing");
+    for (uint64_t b = 0; b < n_blocks; ++b)
+        if (block_offsets[b + 1] - block_offsets[b] > 2u * kBlock)
+            return fail_msg(SNAPPY_B200_ERR_FRAMING, "a block is longer than the block decoders take (2 * 65536 stream bytes)");
     const int G = (int)std::min<uint64_t>(usable_devices(n_devices), n_blocks);
     if (G < 1)
         return fail_msg(SNAPPY_B200_ERR_CUDA, "no usable CUDA device");
@@ -345,6 +348,19 @@ int snappy_b200_decompress_host_indexed_multi(const void *stream, uint64_t strea
         return rc;
     *out_bytes = total;
     return SNAPPY_B200_OK;
+}
+
+int snappy_b200_decompress_host_indexed_multi(const void *stream, uint64_t stream_bytes, const uint64_t *block_offsets,
+                                              uint64_t n_blocks, void *out, uint64_t out_capacity, uint64_t *out_bytes,
+                                              int n_devices)
+{
+    const int rc = decompress_host_indexed_multi_blocks(stream, stream_bytes, block_offsets, n_blocks, out, out_capacity,
+                                                        out_bytes, n_devices);
+    if (rc != SNAPPY_B200_ERR_FRAMING)
+        return rc;
+    // valid raw Snappy the block decoders do not take: the general decoder on the current device
+    clear_error();
+    return decompress_host_general(stream, stream_bytes, out, out_bytes); // (all arguments were checked above)
 }
 
 int snappy_b200_decompress_host_multi(const void *stream, uint64_t stream_bytes, void *out, uint64_t out_capacity,
@@ -397,9 +413,13 @@ int snappy_b200_decompress_host_multi(const void *stream, uint64_t stream_bytes,
         };
         k0();
         rc = finish(std::vector<Result>{r});
-        if (rc != SNAPPY_B200_OK)
-            return rc;
     }
+    if (rc == SNAPPY_B200_ERR_FRAMING) { // an element straddles a block: the general decoder on the current device
+        clear_error();
+        return decompress_host_general(stream, stream_bytes, out, out_bytes);
+    }
+    if (rc != SNAPPY_B200_OK)
+        return rc;
     return snappy_b200_decompress_host_indexed_multi(stream, stream_bytes, offs.data(), nb, out, out_capacity, out_bytes,
                                                      n_devices);
 }
