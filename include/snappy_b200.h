@@ -54,12 +54,14 @@ extern "C" {
 #define SNAPPY_B200_ERR_CORRUPT (-4)  /* malformed compressed stream */
 #define SNAPPY_B200_ERR_FRAMING (-5)  /* valid Snappy, but an element straddles a 64 KiB block */
 #define SNAPPY_B200_ERR_IO (-6)       /* FILE* read/write failed (drop-in layer) */
+#define SNAPPY_B200_ERR_CHECKSUM (-7) /* framed stream: a chunk's CRC-32C does not match its data */
 
 /* Status word written by the device kernels (bit set; 0 = clean). */
 #define SNAPPY_B200_ST_CAPACITY 1u
 #define SNAPPY_B200_ST_CORRUPT 2u
 #define SNAPPY_B200_ST_FRAMING 4u
 #define SNAPPY_B200_ST_UNRESOLVED 8u /* the element chain did not resolve within the relaxation rounds run */
+#define SNAPPY_B200_ST_CHECKSUM 16u  /* framed stream: a chunk's CRC-32C does not match (CORRUPT takes precedence) */
 
 /* Message of the last failing call on this thread (never NULL). */
 const char *snappy_b200_last_error(void);
@@ -196,6 +198,52 @@ int snappy_b200_decompress_file_indexed(FILE *in, FILE *index_in, FILE *out);
  * page-locked 32 MiB chunks on the host (fread -> H2D, K0 + decode, D2H -> fwrite).  Returns 1 (nothing read,
  * nothing written) when `in` is not seekable or the data does not fit the device: decode whole buffers then. */
 int snappy_b200_decompress_file(FILE *in, FILE *out);
+/* ---------------------------------------------------------------- framing format
+ * The Snappy framing format of google/snappy framing_format.txt (".sz" files; what golang/snappy, the Rust `snap`
+ * crate and python-snappy read and write): the stream identifier ff 06 00 00 "sNaPpY", then chunks of a 1-byte type
+ * and a 3-byte little-endian length.  A data chunk carries at most 65536 uncompressed bytes and the masked CRC-32C
+ * (Castagnoli; ((c >> 15) | (c << 17)) + 0xa282ead8, little-endian) of them: 0x00 = a raw Snappy buffer
+ * varint(n) || elements whose copies stay inside the chunk, 0x01 = the bytes themselves.  0xff repeats the
+ * identifier, 0xfe (padding) and 0x80-0xfd are skipped, 0x02-0x7f are an error.  Every CRC is checked on decode.
+ *
+ * The writer emits the identifier, then one chunk per 64 KiB block of input (the last may be shorter): compressed
+ * when the raw payload varint(n_b) + the block's elements is shorter than n_b - n_b / 8, uncompressed otherwise
+ * (golang/snappy's rule).  The compressed payload of a block is exactly what snappy_b200_compress_host gives for
+ * that block alone, in either mode.  An empty input gives the identifier alone; an empty buffer decodes as an empty
+ * stream.  SNAPPY_B200_DEVICES does not apply: the framed calls run on the current device.                        */
+
+/* Upper bound of a framed stream for n input bytes: 10 + n + 8 * ceil(n / 65536). */
+uint64_t snappy_b200_frame_max_compressed_bytes(uint64_t n_bytes);
+size_t snappy_b200_frame_compress_workspace_bytes(uint64_t n_bytes, int mode);
+/* Device-level framed compression: d_in / d_out / d_workspace as for snappy_b200_compress_device (16-byte
+ * aligned; the workspace is required, also for n_bytes == 0).  *d_out_bytes receives the stream length, *d_status
+ * SNAPPY_B200_ST_* bits (CAPACITY when out_capacity was too small).  Enqueue only: no read-back, no lock, no
+ * allocation, so the call may be captured into a CUDA graph.                                                      */
+int snappy_b200_frame_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode, uint8_t *d_out,
+                                      uint64_t out_capacity, uint64_t *d_out_bytes, uint32_t *d_status,
+                                      void *d_workspace, size_t workspace_bytes, void *stream);
+/* Host buffers, synchronous, like snappy_b200_compress_host (128 MiB chunks, uploads and downloads overlapped). */
+int snappy_b200_frame_compress_host(const void *in, uint64_t n_bytes, int mode, void *out, uint64_t out_capacity,
+                                    uint64_t *out_bytes);
+/* Host only, no device needed: walks the chunk headers and checks every rule above except the compressed payloads
+ * and the CRCs; *n_bytes = the total uncompressed length.  SNAPPY_B200_ERR_CORRUPT names the offset of the first
+ * bad chunk.                                                                                                     */
+int snappy_b200_frame_uncompressed_length(const void *stream, uint64_t stream_bytes, uint64_t *n_bytes);
+/* Decodes a framed stream from host memory: the chunk headers are walked on the host, the stream goes up in
+ * pieces cut at chunk boundaries, every piece is decoded (one warp per chunk, no K0) and checked (CRC-32C of every
+ * chunk) while the next one is in flight.  SNAPPY_B200_ERR_CORRUPT for a malformed stream,
+ * SNAPPY_B200_ERR_CHECKSUM when the stream is well formed but a chunk's data does not match its CRC.            */
+int snappy_b200_frame_decompress_host(const void *stream, uint64_t stream_bytes, void *out, uint64_t out_capacity,
+                                      uint64_t *out_bytes);
+/* FILE* -> FILE* (the command line's `-f`; caller opens and closes).  Compression reads the input in chunks of
+ * whole blocks through a ring of page-locked buffers (reader thread -> GPU -> writer thread), as the drop-in
+ * snappy_compress does; an empty input gives the identifier alone.  Decompression needs no seekable input: it
+ * reads 32 MiB windows, decodes the chunks that are complete in each (at most 32 MiB of output at a time) and
+ * carries the incomplete tail into the next window, so page-locked and device memory are bounded by the window
+ * size, not by the file size.                                                                                    */
+int snappy_b200_frame_compress_file(FILE *in, FILE *out, int mode);
+int snappy_b200_frame_decompress_file(FILE *in, FILE *out);
+
 /* Releases the cached device/pinned buffers of the host-buffer API. */
 void snappy_b200_release(void);
 /* Page-locked host memory for the buffers handed to the host-buffer API (what the reference's

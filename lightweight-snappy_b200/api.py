@@ -28,7 +28,8 @@ BLOCK = 65536
 SLOT_STRIDE = 66560
 MODE_HASH, MODE_BST = 0, 1
 OK = 0
-ST_CAPACITY, ST_CORRUPT, ST_FRAMING = 1, 2, 4
+ERR_CUDA, ERR_ARG, ERR_CAPACITY, ERR_CORRUPT, ERR_FRAMING, ERR_IO, ERR_CHECKSUM = -1, -2, -3, -4, -5, -6, -7
+ST_CAPACITY, ST_CORRUPT, ST_FRAMING, ST_CHECKSUM = 1, 2, 4, 16
 
 _u8p = C.c_void_p
 
@@ -74,6 +75,15 @@ SIGNATURES = {
     "snappy_b200_decompress_file": (C.c_int, [C.c_void_p, C.c_void_p]),
     "snappy_b200_compress_file_indexed": (C.c_int, [C.c_void_p, C.c_ulonglong, C.c_int, C.c_void_p, C.c_void_p]),
     "snappy_b200_decompress_file_indexed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "snappy_b200_frame_max_compressed_bytes": (C.c_uint64, [C.c_uint64]),
+    "snappy_b200_frame_compress_workspace_bytes": (C.c_size_t, [C.c_uint64, C.c_int]),
+    "snappy_b200_frame_compress_device": (C.c_int, [_u8p, C.c_uint64, C.c_int, _u8p, C.c_uint64, _u8p, _u8p, _u8p,
+                                                    C.c_size_t, C.c_void_p]),
+    "snappy_b200_frame_compress_host": (C.c_int, [_u8p, C.c_uint64, C.c_int, _u8p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "snappy_b200_frame_uncompressed_length": (C.c_int, [_u8p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "snappy_b200_frame_decompress_host": (C.c_int, [_u8p, C.c_uint64, _u8p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    "snappy_b200_frame_compress_file": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int]),
+    "snappy_b200_frame_decompress_file": (C.c_int, [C.c_void_p, C.c_void_p]),
     "snappy_b200_release": (None, []),
     "snappy_b200_host_alloc": (C.c_void_p, [C.c_size_t]),
     "snappy_b200_host_free": (None, [C.c_void_p]),
@@ -232,6 +242,35 @@ def snappy_decompress(stream) -> np.ndarray:
     return decompress_host(stream)
 
 
+# ------------------------------------------------------------------ framing format (.sz, framing_format.txt)
+def compress_framed(data, mode: int = MODE_HASH) -> np.ndarray:
+    """A framed stream: the stream identifier, then one CRC-checked chunk per 64 KiB block."""
+    a = _host_u8(data)
+    out = np.empty(int(lib().snappy_b200_frame_max_compressed_bytes(a.size)), dtype=np.uint8)
+    n = C.c_uint64(0)
+    _check(lib().snappy_b200_frame_compress_host(a.ctypes.data, a.size, mode, out.ctypes.data, out.size, C.byref(n)))
+    return out[: n.value]
+
+
+def framed_uncompressed_length(stream) -> int:
+    """Total uncompressed length of a framed stream; walks the chunk headers on the host (no device needed)."""
+    a = _host_u8(stream)
+    n = C.c_uint64(0)
+    _check(lib().snappy_b200_frame_uncompressed_length(a.ctypes.data, a.size, C.byref(n)))
+    return n.value
+
+
+def decompress_framed(stream, out: np.ndarray | None = None) -> np.ndarray:
+    """Decodes a framed stream; SnappyError with code ERR_CHECKSUM when a chunk's CRC-32C does not match."""
+    a = _host_u8(stream)
+    total = framed_uncompressed_length(a)
+    if out is None:
+        out = np.empty(max(total, 1), dtype=np.uint8)
+    n = C.c_uint64(0)
+    _check(lib().snappy_b200_frame_decompress_host(a.ctypes.data, a.size, out.ctypes.data, out.size, C.byref(n)))
+    return out[: n.value]
+
+
 # ------------------------------------------------------------------ device-level API (torch)
 class DeviceCodec:
     """Pre-allocated device buffers for repeated device-resident calls on one size class.
@@ -253,7 +292,8 @@ class DeviceCodec:
         ws = max(int(L.snappy_b200_compress_workspace_bytes(max_bytes, MODE_BST)),
                  int(L.snappy_b200_index_workspace_bytes(self.comp_capacity)),
                  int(L.snappy_b200_decompress_workspace_bytes(self.comp_capacity, max_bytes)),
-                 int(L.snappy_b200_decompress_async_workspace_bytes(self.comp_capacity, max_bytes)))
+                 int(L.snappy_b200_decompress_async_workspace_bytes(self.comp_capacity, max_bytes)),
+                 int(L.snappy_b200_frame_compress_workspace_bytes(max_bytes, MODE_BST)))
         self.workspace = torch.empty(ws + 256, dtype=torch.uint8, device=self.device)
         self.stream_buf = torch.empty(self.comp_capacity + 256, dtype=torch.uint8, device=self.device)
         self.block_offsets = torch.zeros(nb + 1, dtype=torch.int64, device=self.device)
@@ -271,6 +311,14 @@ class DeviceCodec:
             data.data_ptr(), n, mode, self.stream_buf.data_ptr(), self.comp_capacity, self.out_bytes.data_ptr(),
             self.block_offsets.data_ptr(), self.status.data_ptr(), self.workspace.data_ptr(),
             self.workspace.numel(), self._stream()))
+
+    def compress_framed(self, data, mode: int = MODE_HASH):
+        """data: uint8 CUDA tensor.  A framed stream into stream_buf / out_bytes / status (enqueue only)."""
+        n = data.numel()
+        assert data.is_cuda and data.dtype == self.torch.uint8 and data.is_contiguous() and n <= self.max_bytes
+        _check(lib().snappy_b200_frame_compress_device(
+            data.data_ptr(), n, mode, self.stream_buf.data_ptr(), self.stream_buf.numel(), self.out_bytes.data_ptr(),
+            self.status.data_ptr(), self.workspace.data_ptr(), self.workspace.numel(), self._stream()))
 
     def decompress_indexed(self, stream_t, block_offsets, total_out: int, out):
         """Decodes with a known block index (e.g. the one compress() produced)."""

@@ -25,6 +25,8 @@ cudaError_t run_index(const uint8_t *, uint64_t, uint64_t, uint64_t, uint64_t *,
                       uint64_t *, bool, uint64_t, uint32_t fixed_rounds = 0);
 uint32_t host_varint_len(uint64_t);
 uint64_t index_last_rounds();
+cudaError_t launch_frame_compact(const uint8_t *, uint64_t, const uint8_t *, const uint32_t *, uint32_t *, uint32_t *, int,
+                                 uint8_t *, uint64_t, uint64_t *, uint64_t *, uint32_t *, cudaStream_t, uint64_t *);
 
 static thread_local char g_err[512] = "";
 static std::atomic<uint64_t> g_launches{0};
@@ -74,6 +76,21 @@ static CompressWorkspace carve_compress(void *ws, uint64_t n_bytes)
     return w;
 }
 
+// The framed compressor's workspace: the raw compressor's, then the masked CRC and the chunk size of every block.
+static size_t frame_ws_bytes(uint64_t n_bytes)
+{
+    const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
+    return compress_ws_bytes(n_bytes) + 2 * align_up(nb * 4 + 4, 256);
+}
+
+static void carve_frame(void *ws, uint64_t n_bytes, uint32_t **crcs, uint32_t **fsizes)
+{
+    const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
+    uint8_t *p = static_cast<uint8_t *>(ws) + compress_ws_bytes(n_bytes);
+    *crcs = reinterpret_cast<uint32_t *>(p);
+    *fsizes = reinterpret_cast<uint32_t *>(p + align_up(nb * 4 + 4, 256));
+}
+
 static int status_to_error(uint32_t st)
 {
     // FRAMING first: once an element leaves the 64 KiB framing the blocks after it may look malformed to the
@@ -84,6 +101,8 @@ static int status_to_error(uint32_t st)
                     "earlier one; device status 0x%x)", st);
     if (st & SNAPPY_B200_ST_CORRUPT)
         return fail(SNAPPY_B200_ERR_CORRUPT, "malformed compressed stream (device status 0x%x)", st);
+    if (st & SNAPPY_B200_ST_CHECKSUM)
+        return fail(SNAPPY_B200_ERR_CHECKSUM, "a chunk's CRC-32C does not match its data (device status 0x%x)", st);
     if (st & SNAPPY_B200_ST_UNRESOLVED)
         return fail(SNAPPY_B200_ERR_CORRUPT,
                     "the element chain of the stream did not resolve within the relaxation rounds allowed "
@@ -100,7 +119,10 @@ int fail_msg(int code, const char *msg) { return fail(code, "%s", msg); }
 void clear_error() { g_err[0] = 0; } // every public entry point starts clean: a stale message is never reported twice
 int cuda_fail_msg(cudaError_t e, const char *what) { return cuda_fail(e, what); }
 int status_error(uint32_t st) { return status_to_error(st); }
-size_t compress_workspace_bytes_internal(uint64_t n_bytes) { return compress_ws_bytes(n_bytes); }
+size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed)
+{
+    return framed ? frame_ws_bytes(n_bytes) : compress_ws_bytes(n_bytes);
+}
 void add_launches(uint64_t n) { g_launches += n; }
 
 // Small device -> host read-backs (sizes, flags, status words).  A cudaMemcpyAsync would queue
@@ -131,19 +153,27 @@ uint32_t *thread_pinned_scratch()
     return p;
 }
 
-// One chunk of a longer input: blocks only, or (first chunk) the varint of the WHOLE input
-// followed by blocks.  Same kernels as snappy_b200_compress_device.
-cudaError_t compress_chunk(const uint8_t *d_in, uint64_t chunk_bytes, uint64_t varint_value, int mode, uint8_t *d_out,
-                           uint64_t out_capacity, uint64_t *d_out_bytes, uint32_t *d_status, void *d_workspace,
-                           cudaStream_t st)
+// One chunk of a longer input: blocks only, or (varint_value != 0: the chunk opens the stream) the varint of the
+// WHOLE input followed by blocks.  framed: data chunks of the framing format instead of bare blocks (varint_value
+// is not used), with the stream identifier in front when `identifier` is set.  Same kernels as
+// snappy_b200_compress_device / snappy_b200_frame_compress_device.
+cudaError_t compress_chunk(const uint8_t *d_in, uint64_t chunk_bytes, uint64_t varint_value, int mode, bool framed,
+                           bool identifier, uint8_t *d_out, uint64_t out_capacity, uint64_t *d_out_bytes,
+                           uint32_t *d_status, void *d_workspace, cudaStream_t st)
 {
     const uint64_t nb = (chunk_bytes + kBlock - 1) / kBlock;
     CompressWorkspace w = carve_compress(d_workspace, chunk_bytes);
     uint64_t launches = 0;
     cudaError_t e = launch_compress(d_in, chunk_bytes, mode, w.scratch, w.sizes, w.recs, w.nrec, st, &launches);
-    if (e == cudaSuccess)
+    if (e == cudaSuccess && framed) {
+        uint32_t *crcs, *fsizes;
+        carve_frame(d_workspace, chunk_bytes, &crcs, &fsizes);
+        e = launch_frame_compact(d_in, chunk_bytes, w.scratch, w.sizes, crcs, fsizes, identifier ? 1 : 0, d_out,
+                                 out_capacity, w.offsets, d_out_bytes, d_status, st, &launches);
+    } else if (e == cudaSuccess) {
         e = launch_compact(w.scratch, w.sizes, nb, varint_value, varint_value ? host_varint_len(varint_value) : 0,
                            varint_value ? 1 : 0, d_out, out_capacity, w.offsets, d_out_bytes, d_status, st, &launches);
+    }
     g_launches += launches;
     return e;
 }
@@ -221,6 +251,42 @@ int snappy_b200_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode,
     g_launches += launches;
     if (e != cudaSuccess)
         return cuda_fail(e, "compress launch");
+    return SNAPPY_B200_OK;
+}
+
+uint64_t snappy_b200_frame_max_compressed_bytes(uint64_t n_bytes)
+{
+    return 10 + n_bytes + 8 * snappy_b200_block_count(n_bytes);
+}
+
+size_t snappy_b200_frame_compress_workspace_bytes(uint64_t n_bytes, int mode)
+{
+    (void)mode;
+    return frame_ws_bytes(n_bytes);
+}
+
+int snappy_b200_frame_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode, uint8_t *d_out,
+                                      uint64_t out_capacity, uint64_t *d_out_bytes, uint32_t *d_status,
+                                      void *d_workspace, size_t workspace_bytes, void *stream)
+{
+    clear_error();
+    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
+        return fail(SNAPPY_B200_ERR_ARG, "unknown mode %d", mode);
+    if (!d_out_bytes || !d_status || !d_out || !d_workspace || (n_bytes && !d_in))
+        return fail(SNAPPY_B200_ERR_ARG, "null pointer argument");
+    if (!aligned16(d_in) || !aligned16(d_out) || !aligned16(d_workspace))
+        return fail(SNAPPY_B200_ERR_ARG, "d_in, d_out and d_workspace must be 16-byte aligned");
+    if (workspace_bytes < frame_ws_bytes(n_bytes))
+        return fail(SNAPPY_B200_ERR_ARG, "workspace too small: %zu < %zu", workspace_bytes, frame_ws_bytes(n_bytes));
+    if ((n_bytes + kBlock - 1) / kBlock > 0x7fffffffull)
+        return fail(SNAPPY_B200_ERR_ARG, "input too large");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    cudaError_t e = cudaMemsetAsync(d_status, 0, sizeof(uint32_t), st);
+    if (e != cudaSuccess)
+        return cuda_fail(e, "cudaMemsetAsync(status)");
+    e = compress_chunk(d_in, n_bytes, 0, mode, true, true, d_out, out_capacity, d_out_bytes, d_status, d_workspace, st);
+    if (e != cudaSuccess)
+        return cuda_fail(e, "framed compress launch");
     return SNAPPY_B200_OK;
 }
 

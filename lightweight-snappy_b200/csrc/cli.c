@@ -18,13 +18,15 @@
 
 static void usage(void)
 {
-    fprintf(stderr, "snappy [-c|-d|-b] [-r] [-i] [infile] [outfile]\n"
+    fprintf(stderr, "snappy [-c|-d|-b] [-r] [-i|-f] [infile] [outfile]\n"
                     "-c compress (hash table)\n"
                     "-b compress (exact-key / BST match finder)\n"
                     "-d decompress\n"
                     "-r print sizes, ratio, time and throughput\n"
                     "-i side index: compress also writes <outfile>.idx (block offsets; the stream is\n"
-                    "   unchanged), decompress reads <infile>.idx and skips the boundary search\n");
+                    "   unchanged), decompress reads <infile>.idx and skips the boundary search\n"
+                    "-f the Snappy framing format (.sz: stream identifier, CRC-32C-checked chunks) instead of\n"
+                    "   the reference's stream; the input of -d may be a pipe\n");
     exit(EXIT_FAILURE);
 }
 
@@ -46,18 +48,23 @@ static double now(void)
 int main(int argc, char *argv[])
 {
     enum { COMPRESS, COMPRESS_BST, UNCOMPRESS } mode = COMPRESS;
-    int report = 0, use_index = 0, opt;
+    int report = 0, use_index = 0, framed = 0, opt;
     if (argc < 4)
         usage();
-    while ((opt = getopt(argc, argv, "cbdri")) != -1) {
+    while ((opt = getopt(argc, argv, "cbdrif")) != -1) {
         switch (opt) {
         case 'c': mode = COMPRESS; break;
         case 'b': mode = COMPRESS_BST; break;
         case 'd': mode = UNCOMPRESS; break;
         case 'r': report = 1; break;
         case 'i': use_index = 1; break;
+        case 'f': framed = 1; break;
         default: usage();
         }
+    }
+    if (framed && use_index) {
+        fprintf(stderr, "-f and -i cannot be combined: the chunk headers of a framed stream are its index\n");
+        usage();
     }
     const char *in_name = argv[argc - 2], *out_name = argv[argc - 1];
     FILE *in = fopen(in_name, "rb");
@@ -71,7 +78,7 @@ int main(int argc, char *argv[])
         fclose(in);
         return EXIT_FAILURE;
     }
-    const unsigned long long in_size = file_size(in);
+    const unsigned long long in_size = framed && mode == UNCOMPRESS ? 0 : file_size(in); /* (-f -d: may be a pipe) */
     int rc = 0;
     FILE *idx = NULL;
     if (use_index) {
@@ -86,7 +93,11 @@ int main(int argc, char *argv[])
         }
     }
     const double t0 = now();
-    if (idx && mode == UNCOMPRESS)
+    if (framed && mode == UNCOMPRESS)
+        rc = snappy_b200_frame_decompress_file(in, out);
+    else if (framed)
+        rc = snappy_b200_frame_compress_file(in, out, mode == COMPRESS ? SNAPPY_B200_MODE_HASH : SNAPPY_B200_MODE_BST);
+    else if (idx && mode == UNCOMPRESS)
         rc = snappy_b200_decompress_file_indexed(in, idx, out);
     else if (idx)
         rc = snappy_b200_compress_file_indexed(in, in_size, mode == COMPRESS ? SNAPPY_B200_MODE_HASH : SNAPPY_B200_MODE_BST,

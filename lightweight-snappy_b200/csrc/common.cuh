@@ -14,6 +14,17 @@ constexpr unsigned kFull = 0xffffffffu;
 constexpr uint32_t kHashMul = 0x1e35a7bdu;  // reference: src/snappy_compression.c:82
 constexpr uint32_t kAbortMark = 0xffffffffu; // sizes[] entry of a block a table tier gave up on
 
+// ---- framed streams (csrc/frame.cu): one data chunk, as the host walk of the chunk headers describes it
+constexpr uint32_t kChunkCompressed = 0x00, kChunkUncompressed = 0x01;
+struct FrameChunk {
+    uint64_t in_off;   // stream offset of the chunk's body: the elements (after the varint), or the raw bytes
+    uint64_t out_off;  // output offset of its first byte
+    uint32_t in_len;   // body bytes
+    uint32_t out_len;  // uncompressed bytes, <= 65536
+    uint32_t type;     // kChunkCompressed / kChunkUncompressed
+    uint32_t crc;      // the stored (masked) CRC-32C
+};
+
 // ---- read-only input access -------------------------------------------------------------
 // `base` is 4-byte aligned.  Word `last_word` is the last one that holds a valid byte, so the
 // second load is clamped instead of running past the buffer when pos is word aligned.

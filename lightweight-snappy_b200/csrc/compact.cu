@@ -129,6 +129,16 @@ cudaError_t launch_compact(const uint8_t *d_scratch, const uint32_t *d_sizes, ui
     return cudaGetLastError();
 }
 
+cudaError_t launch_scan_sizes(const uint32_t *d_sizes, uint64_t n_blocks, uint64_t n_bytes, uint64_t base,
+                              int write_varint, uint8_t *d_out, uint64_t out_capacity, uint64_t *d_offsets,
+                              uint64_t *d_out_bytes, uint32_t *d_status, cudaStream_t st, uint64_t *launches)
+{
+    k_scan_sizes<<<1, kScanThreads, 0, st>>>(d_sizes, n_blocks, n_bytes, base, write_varint, d_out, out_capacity,
+                                             d_offsets, d_out_bytes, d_status);
+    *launches += 1;
+    return cudaGetLastError();
+}
+
 uint32_t host_varint_len(uint64_t v) { return varint_len(v); }
 
 } // namespace sb200

@@ -493,32 +493,13 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
 }
 
 // ------------------------------------------------------------------ window decoder (block index only)
-__global__ void __launch_bounds__(32) k_decode_warp(const uint8_t *__restrict__ stream,
-                                                    const uint64_t *__restrict__ offsets, uint64_t total_out,
-                                                    uint8_t *out_base, uint32_t *__restrict__ status)
+// One compressed block of clen stream bytes at `in` into olen output bytes at `out`, by one warp.  `elems` is the
+// warp's 32-entry shared table; `last_word` clamps the loads to the stream.  Returns an error status or 0.
+// `blk` only tells ST_CORRUPT from ST_FRAMING for a copy that reaches before the block.
+__device__ __forceinline__ uint32_t decode_block_warp(const uint8_t *__restrict__ in, uint32_t clen,
+                                                      const uint32_t *__restrict__ last_word, uint8_t *out, uint32_t olen,
+                                                      uint64_t blk, uint4 *elems, uint32_t lane)
 {
-    __shared__ uint4 elems[32];
-    const uint32_t lane = threadIdx.x;
-    const uint64_t blk = blockIdx.x;
-    if (*reinterpret_cast<volatile uint32_t *>(status) != 0)
-        return; // an earlier stage rejected the stream: the offsets are not trustworthy
-    const uint64_t c0 = offsets[blk], c1 = offsets[blk + 1];
-    const uint64_t stream_bytes = offsets[gridDim.x]; // entry n_blocks of the index = end of the stream
-    const uint64_t clen64 = c1 - c0;
-    if (c1 < c0 || c1 > stream_bytes || clen64 > 2u * kBlock) { // a compressor's block never needs more than 65536+1010
-        // a longer block is valid raw Snappy (non-minimal encodings) that only the general decoder takes
-        if (lane == 0)
-            atomicOr(status, c1 < c0 || c1 > stream_bytes ? SNAPPY_B200_ST_CORRUPT : SNAPPY_B200_ST_FRAMING);
-        return;
-    }
-    const uint8_t *__restrict__ in = stream + c0;
-    const uint32_t *last_word = reinterpret_cast<const uint32_t *>(
-        reinterpret_cast<uintptr_t>(stream + stream_bytes - 1) & ~uintptr_t(3));
-    uint8_t *out = out_base + blk * (uint64_t)kBlock;
-    const uint64_t oleft = total_out - blk * (uint64_t)kBlock;
-    const uint32_t olen = oleft < kBlock ? (uint32_t)oleft : kBlock;
-    const uint32_t clen = (uint32_t)clen64;
-
     uint32_t ip = 0, op = 0;
     uint32_t err = 0;
     while (op < olen && !err) {
@@ -573,6 +554,34 @@ __global__ void __launch_bounds__(32) k_decode_warp(const uint8_t *__restrict__ 
     }
     if (!err && ip != clen)
         err = SNAPPY_B200_ST_CORRUPT; // the index said this block ends at c1
+    return err;
+}
+
+__global__ void __launch_bounds__(32) k_decode_warp(const uint8_t *__restrict__ stream,
+                                                    const uint64_t *__restrict__ offsets, uint64_t total_out,
+                                                    uint8_t *out_base, uint32_t *__restrict__ status)
+{
+    __shared__ uint4 elems[32];
+    const uint32_t lane = threadIdx.x;
+    const uint64_t blk = blockIdx.x;
+    if (*reinterpret_cast<volatile uint32_t *>(status) != 0)
+        return; // an earlier stage rejected the stream: the offsets are not trustworthy
+    const uint64_t c0 = offsets[blk], c1 = offsets[blk + 1];
+    const uint64_t stream_bytes = offsets[gridDim.x]; // entry n_blocks of the index = end of the stream
+    const uint64_t clen64 = c1 - c0;
+    if (c1 < c0 || c1 > stream_bytes || clen64 > 2u * kBlock) { // a compressor's block never needs more than 65536+1010
+        // a longer block is valid raw Snappy (non-minimal encodings) that only the general decoder takes
+        if (lane == 0)
+            atomicOr(status, c1 < c0 || c1 > stream_bytes ? SNAPPY_B200_ST_CORRUPT : SNAPPY_B200_ST_FRAMING);
+        return;
+    }
+    const uint8_t *__restrict__ in = stream + c0;
+    const uint32_t *last_word = reinterpret_cast<const uint32_t *>(
+        reinterpret_cast<uintptr_t>(stream + stream_bytes - 1) & ~uintptr_t(3));
+    uint8_t *out = out_base + blk * (uint64_t)kBlock;
+    const uint64_t oleft = total_out - blk * (uint64_t)kBlock;
+    const uint32_t olen = oleft < kBlock ? (uint32_t)oleft : kBlock;
+    const uint32_t err = decode_block_warp(in, (uint32_t)clen64, last_word, out, olen, blk, elems, lane);
     if (err && lane == 0)
         atomicOr(status, err);
 }
@@ -584,12 +593,13 @@ __global__ void __launch_bounds__(32) k_decode_warp(const uint8_t *__restrict__ 
 // decoders report such streams as ST_FRAMING; this kernel then decodes them the way the reference does, one
 // element after the other over the whole output, with one warp moving the bytes of each element.  It is a
 // correctness fallback for rare foreign streams (about an element per microsecond), not a fast path.
-__global__ void __launch_bounds__(32) k_decode_sequential(const uint8_t *__restrict__ stream, uint64_t stream_bytes,
-                                                          uint64_t body_offset, uint64_t total_out, uint8_t *out,
-                                                          uint32_t *__restrict__ status)
+// The element loop over stream bytes [ip, stream_bytes) into total_out bytes at `out`, one warp; copies reach at
+// most back to out[0].  Returns an error status or 0.
+__device__ __forceinline__ uint32_t decode_sequential_warp(const uint8_t *__restrict__ stream, uint64_t ip,
+                                                           uint64_t stream_bytes, uint8_t *out, uint64_t total_out,
+                                                           uint32_t lane)
 {
-    const uint32_t lane = threadIdx.x;
-    uint64_t ip = body_offset, op = 0;
+    uint64_t op = 0;
     uint32_t err = 0;
     while (op < total_out) {
         if (ip >= stream_bytes) {
@@ -636,6 +646,15 @@ __global__ void __launch_bounds__(32) k_decode_sequential(const uint8_t *__restr
     }
     if (!err && ip != stream_bytes)
         err = SNAPPY_B200_ST_CORRUPT; // trailing bytes after the declared length
+    return err;
+}
+
+__global__ void __launch_bounds__(32) k_decode_sequential(const uint8_t *__restrict__ stream, uint64_t stream_bytes,
+                                                          uint64_t body_offset, uint64_t total_out, uint8_t *out,
+                                                          uint32_t *__restrict__ status)
+{
+    const uint32_t lane = threadIdx.x;
+    const uint32_t err = decode_sequential_warp(stream, body_offset, stream_bytes, out, total_out, lane);
     if (err && lane == 0)
         atomicOr(status, err);
 }
@@ -659,6 +678,46 @@ cudaError_t launch_decode(const uint8_t *d_stream, const uint64_t *d_offsets, ui
     if (n_blocks > 0x7fffffffull)
         return cudaErrorInvalidValue;
     k_decode_warp<<<(unsigned)n_blocks, 32, 0, st>>>(d_stream, d_offsets, total_out, d_out, d_status);
+    *launches += 1;
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------ framed streams (csrc/frame.cu)
+// One warp per data chunk of a framed stream.  A chunk is self-contained, so any error -- also what the block
+// routine calls ST_FRAMING (a copy before the chunk, output past its length) -- is ST_CORRUPT here.  A compressed
+// body longer than the window decoder takes (non-minimal encodings: up to 6 stream bytes per output byte) goes
+// through the element loop of the general decoder, so a valid framed stream never needs a host fallback.
+__global__ void __launch_bounds__(32) k_frame_decode(const uint8_t *__restrict__ stream, uint64_t stream_bytes,
+                                                     const FrameChunk *__restrict__ chunks, uint8_t *out_base,
+                                                     uint32_t *__restrict__ status)
+{
+    __shared__ uint4 elems[32];
+    const uint32_t lane = threadIdx.x;
+    const FrameChunk c = chunks[blockIdx.x];
+    uint8_t *out = out_base + c.out_off;
+    const uint8_t *__restrict__ in = stream + c.in_off;
+    uint32_t err = 0;
+    if (c.type == kChunkUncompressed) {
+        coop_copy_ro(out, in, c.out_len, lane, 32);
+    } else if (c.in_len <= 2u * kBlock) {
+        const uint32_t *last_word = reinterpret_cast<const uint32_t *>(
+            reinterpret_cast<uintptr_t>(stream + stream_bytes - 1) & ~uintptr_t(3));
+        err = decode_block_warp(in, c.in_len, last_word, out, c.out_len, 0, elems, lane);
+    } else {
+        err = decode_sequential_warp(in, 0, c.in_len, out, c.out_len, lane);
+    }
+    if (err && lane == 0)
+        atomicOr(status, SNAPPY_B200_ST_CORRUPT);
+}
+
+cudaError_t launch_frame_decode(const uint8_t *d_stream, uint64_t stream_bytes, const FrameChunk *d_chunks,
+                                uint64_t n_chunks, uint8_t *d_out, uint32_t *d_status, cudaStream_t st, uint64_t *launches)
+{
+    if (n_chunks == 0)
+        return cudaSuccess;
+    if (n_chunks > 0x7fffffffull)
+        return cudaErrorInvalidValue;
+    k_frame_decode<<<(unsigned)n_chunks, 32, 0, st>>>(d_stream, stream_bytes, d_chunks, d_out, d_status);
     *launches += 1;
     return cudaGetLastError();
 }

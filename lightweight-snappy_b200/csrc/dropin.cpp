@@ -24,6 +24,8 @@
 namespace sb200 {
 int fail_msg(int code, const char *msg); // abi.cu: records the thread's last error
 void clear_error();
+int frame_compress_host_range(const void *, uint64_t, int, void *, uint64_t, uint64_t *, bool); // host_pipeline.cu
+int frame_decompress_buffer(const void *, uint64_t, void *, uint64_t, uint64_t *, bool);          // host_pipeline.cu
 } // namespace sb200
 
 namespace {
@@ -181,14 +183,18 @@ uint64_t stream_chunk_bytes(unsigned long long declared)
     return chunk;
 }
 
-int compress_file(FILE *in, unsigned long long declared, FILE *out, int mode, FILE *index_out = nullptr)
+// framed: the framing format (stream identifier, then CRC-checked chunks) instead of the reference's stream;
+// `declared` only sizes the chunks then.
+int compress_file(FILE *in, unsigned long long declared, FILE *out, int mode, FILE *index_out = nullptr,
+                  bool framed = false)
 {
     sb200::clear_error();
     if (!in || !out)
         return io_fail("null FILE*");
     constexpr int kInFlight = 3;
     const uint64_t chunk = stream_chunk_bytes(declared);
-    const uint64_t out_cap = snappy_b200_max_compressed_bytes(chunk);
+    const uint64_t out_cap =
+        framed ? snappy_b200_frame_max_compressed_bytes(chunk) : snappy_b200_max_compressed_bytes(chunk);
     PinnedBuf ibuf[kInFlight], obuf[kInFlight];
     uint64_t ilen[kInFlight] = {}, olen[kInFlight] = {};
     ChunkQueue free_in, filled, to_write, free_out;
@@ -255,7 +261,7 @@ int compress_file(FILE *in, unsigned long long declared, FILE *out, int mode, FI
         const uint64_t n = ilen[s];
         if (n < chunk)
             ended = true; // the last chunk (possibly empty)
-        if (n == 0) {
+        if (n == 0 && !(framed && first)) { // (an empty input still gets the stream identifier when framed)
             free_in.push(s);
             break;
         }
@@ -266,13 +272,15 @@ int compress_file(FILE *in, unsigned long long declared, FILE *out, int mode, FI
         const uint64_t nb = snappy_b200_block_count(n);
         if (index_out)
             offs.resize(nb + 1);
-        if (rc == SNAPPY_B200_OK)
+        if (rc == SNAPPY_B200_OK && framed)
+            rc = sb200::frame_compress_host_range(ibuf[s].p, n, mode, obuf[o].p, obuf[o].cap, &got, first);
+        else if (rc == SNAPPY_B200_OK)
             // the reference writes the DECLARED size into the preamble (src/snappy_compression.c:417) and then
             // whatever the file really holds: keep that even when the two disagree
             rc = snappy_b200_compress_host_range(ibuf[s].p, n, mode, obuf[o].p, obuf[o].cap, &got,
                                                  index_out ? offs.data() : nullptr,
                                                  first ? (declared ? declared : ~0ull) : 0);
-        if (rc == SNAPPY_B200_OK && first && declared == 0) {
+        if (rc == SNAPPY_B200_OK && !framed && first && declared == 0) {
             // (a declared size of 0 still needs its one-byte preamble "00": ask for any value, then patch it)
             unsigned char tmp[10];
             const unsigned k = parse_to_varint(~0ull, tmp);
@@ -312,9 +320,73 @@ int compress_file(FILE *in, unsigned long long declared, FILE *out, int mode, FI
     return SNAPPY_B200_OK; // (an empty input leaves an empty output, like the reference: SURVEY.md 8c)
 }
 
+// Framed FILE* -> FILE* decompression with bounded memory and no seek: 32 MiB windows are read into a page-locked
+// buffer, the chunks that are complete in it (at most 32 MiB of output at a time) are decoded by the host-buffer
+// path and written out, and the incomplete tail is carried into the next window.  A chunk is shorter than
+// 16 MiB + 4 bytes, so a window always completes at least one.
+int decompress_file_framed(FILE *in, FILE *out)
+{
+    sb200::clear_error();
+    if (!in || !out)
+        return io_fail("null FILE*");
+    constexpr uint64_t kWindow = 32u << 20, kMaxOut = 32u << 20;
+    PinnedBuf ib, ob;
+    if (!ib.reserve(kWindow) || !ob.reserve(kMaxOut))
+        return io_fail("out of host memory for the window buffers");
+    uint64_t have = 0;
+    bool eof = false, first = true;
+    for (;;) {
+        while (!eof && have < kWindow) {
+            const size_t k = fread(ib.p + have, 1, kWindow - have, in);
+            have += k;
+            if (k == 0) {
+                if (ferror(in))
+                    return io_fail("reading the compressed stream failed");
+                eof = true;
+            }
+        }
+        // the complete chunks at the front, at most kMaxOut bytes of output (but always at least one chunk)
+        uint64_t at = 0, produced = 0;
+        while (at + 4 <= have) {
+            const uint8_t *h = ib.p + at;
+            const uint64_t L = h[1] | (uint64_t)h[2] << 8 | (uint64_t)h[3] << 16;
+            if (at + 4 + L > have)
+                break;
+            // (an upper bound of the chunk's output: the decode checks the chunk itself)
+            const uint64_t o = (h[0] == 0x00 || h[0] == 0x01) ? 65536 : 0;
+            if (at > 0 && produced + o > kMaxOut)
+                break;
+            produced += o;
+            at += 4 + L;
+        }
+        if (at == 0 && eof)
+            at = have; // a truncated chunk (or nothing at all): the decode reports it
+        uint64_t got = 0;
+        const int rc = sb200::frame_decompress_buffer(ib.p, at, ob.p, ob.cap, &got, first);
+        if (rc != SNAPPY_B200_OK)
+            return rc;
+        if (got && fwrite(ob.p, 1, got, out) != got)
+            return io_fail("short write of the output");
+        first = false;
+        memmove(ib.p, ib.p + at, have - at);
+        have -= at;
+        if (eof && have == 0)
+            return SNAPPY_B200_OK;
+    }
+}
+
 } // namespace
 
 extern "C" {
+
+int snappy_b200_frame_compress_file(FILE *in, FILE *out, int mode)
+{
+    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
+        return sb200::fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
+    return compress_file(in, 0, out, mode, nullptr, true);
+}
+
+int snappy_b200_frame_decompress_file(FILE *in, FILE *out) { return decompress_file_framed(in, out); }
 
 int snappy_b200_compress_file_indexed(FILE *in, unsigned long long input_size, int mode, FILE *out, FILE *index_out)
 {

@@ -37,10 +37,14 @@ int fail_msg(int code, const char *msg);
 void clear_error();
 int cuda_fail_msg(cudaError_t e, const char *what);
 int status_error(uint32_t st);
-size_t compress_workspace_bytes_internal(uint64_t n_bytes);
+size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed);
 void add_launches(uint64_t n);
-cudaError_t compress_chunk(const uint8_t *, uint64_t, uint64_t, int, uint8_t *, uint64_t, uint64_t *, uint32_t *, void *,
-                           cudaStream_t);
+cudaError_t compress_chunk(const uint8_t *, uint64_t, uint64_t, int, bool, bool, uint8_t *, uint64_t, uint64_t *, uint32_t *,
+                           void *, cudaStream_t);
+cudaError_t launch_frame_decode(const uint8_t *, uint64_t, const FrameChunk *, uint64_t, uint8_t *, uint32_t *,
+                                cudaStream_t, uint64_t *);
+int frame_decompress_buffer(const void *, uint64_t, void *, uint64_t, uint64_t *, bool);
+cudaError_t launch_frame_check(const uint8_t *, const FrameChunk *, uint64_t, uint32_t *, cudaStream_t, uint64_t *);
 size_t index_workspace_bytes(uint64_t);
 cudaError_t run_index(const uint8_t *, uint64_t, uint64_t, uint64_t, uint64_t *, uint32_t *, void *, cudaStream_t,
                       uint64_t *, bool, uint64_t, uint32_t fixed_rounds = 0);
@@ -98,6 +102,69 @@ unsigned host_varint_decode(const uint8_t *p, uint64_t avail, uint64_t *out)
         }
     }
     return 0;
+}
+
+// ---- framing format (include/snappy_b200.h): the chunk headers are walked on the host
+const uint8_t kStreamId[10] = {0xff, 0x06, 0x00, 0x00, 's', 'N', 'a', 'P', 'p', 'Y'};
+
+int frame_fail(int code, uint64_t at, const char *what)
+{
+    char msg[160];
+    snprintf(msg, sizeof msg, "framed stream, chunk at offset %llu: %s", (unsigned long long)at, what);
+    return fail_msg(code, msg);
+}
+
+// Checks every rule of the framing format except the compressed payloads and the CRCs; *total = the uncompressed
+// length; `chunks` (optional) receives one descriptor per data chunk, in stream order.  opens_stream: the buffer is
+// a whole stream (it must begin with the identifier); otherwise it is a run of whole chunks from inside a stream.
+int frame_walk(const uint8_t *p, uint64_t n, bool opens_stream, std::vector<FrameChunk> *chunks, uint64_t *total)
+{
+    *total = 0;
+    if (n == 0)
+        return SNAPPY_B200_OK; // an empty buffer is an empty stream, as for the raw calls
+    if (opens_stream && (n < sizeof kStreamId || memcmp(p, kStreamId, sizeof kStreamId) != 0))
+        return frame_fail(SNAPPY_B200_ERR_CORRUPT, 0, "the stream does not start with the stream identifier");
+    uint64_t at = opens_stream ? sizeof kStreamId : 0, out = 0;
+    while (at < n) {
+        if (n - at < 4)
+            return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "truncated chunk header");
+        const uint32_t type = p[at], L = p[at + 1] | (uint32_t)p[at + 2] << 8 | (uint32_t)p[at + 3] << 16;
+        if (L > n - at - 4)
+            return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "the chunk runs past the end of the stream");
+        const uint8_t *body = p + at + 4;
+        if (type == kChunkCompressed || type == kChunkUncompressed) {
+            if (L < 4)
+                return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "data chunk shorter than its checksum");
+            FrameChunk c;
+            c.type = type;
+            c.crc = body[0] | (uint32_t)body[1] << 8 | (uint32_t)body[2] << 16 | (uint32_t)body[3] << 24;
+            if (type == kChunkCompressed) {
+                uint64_t len = 0;
+                const unsigned vl = host_varint_decode(body + 4, L - 4, &len);
+                if (!vl)
+                    return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "bad varint in a compressed chunk");
+                if (len > kBlock)
+                    return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "compressed chunk of more than 65536 bytes");
+                c.in_off = at + 8 + vl, c.in_len = L - 4 - vl, c.out_len = (uint32_t)len;
+            } else {
+                if (L - 4 > kBlock)
+                    return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "uncompressed chunk of more than 65536 bytes");
+                c.in_off = at + 8, c.in_len = L - 4, c.out_len = L - 4;
+            }
+            c.out_off = out;
+            out += c.out_len;
+            if (chunks)
+                chunks->push_back(c);
+        } else if (type == 0xff) {
+            if (L != 6 || memcmp(body, kStreamId + 4, 6) != 0)
+                return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "bad stream identifier");
+        } else if (type < 0x80) {
+            return frame_fail(SNAPPY_B200_ERR_CORRUPT, at, "reserved unskippable chunk type");
+        } // 0x80-0xfd reserved skippable, 0xfe padding
+        at += 4 + (uint64_t)L;
+    }
+    *total = out;
+    return SNAPPY_B200_OK;
 }
 
 // Cached per-process resources of the synchronous host-buffer entry points.
@@ -429,27 +496,22 @@ int snappy_b200_compress_host_indexed(const void *in, uint64_t n_bytes, int mode
     return snappy_b200_compress_host_range(in, n_bytes, mode, out, out_capacity, out_bytes, block_offsets, n_bytes);
 }
 
-int snappy_b200_compress_host_range(const void *in, uint64_t n_bytes, int mode, void *out, uint64_t out_capacity,
-                                    uint64_t *out_bytes, uint64_t *block_offsets, uint64_t varint_value)
+} // extern "C"
+
+// The chunk loop of the host-buffer compressors: n_bytes > 0 of input, raw blocks (after the varint of
+// varint_value) or, framed, the chunks of the framing format (after the stream identifier when `identifier` is
+// set).  Arguments checked.
+static int compress_host_chunks(const void *in, uint64_t n_bytes, int mode, bool framed, bool identifier, void *out,
+                                uint64_t out_capacity, uint64_t *out_bytes, uint64_t *block_offsets,
+                                uint64_t varint_value)
 {
-    clear_error();
     HostCtx &g_ctx = current_ctx();
-    if (!out_bytes || (n_bytes && (!in || !out)))
-        return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
-    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
-        return fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
-    *out_bytes = 0;
-    if (n_bytes == 0)
-        return SNAPPY_B200_OK; // reference: an empty input gives an empty stream
-    if (env_devices() > 1 && n_bytes >= kMultiMin)
-        return snappy_b200_compress_host_multi_range(in, n_bytes, mode, out, out_capacity, out_bytes, block_offsets,
-                                                     env_devices(), varint_value);
     std::lock_guard<std::mutex> lock(g_ctx.mu);
     CU(g_ctx.init(), "context init");
     const uint64_t chunk = std::min<uint64_t>(kCompressChunk, align_up(n_bytes, kBlock));
     const uint64_t n_chunks = (n_bytes + chunk - 1) / chunk;
-    const uint64_t out_cap_chunk = max_compressed(chunk);
-    const size_t ws_bytes = compress_workspace_bytes_internal(chunk);
+    const uint64_t out_cap_chunk = framed ? snappy_b200_frame_max_compressed_bytes(chunk) : max_compressed(chunk);
+    const size_t ws_bytes = compress_workspace_bytes_internal(chunk, framed);
     const int slots = (int)std::min<uint64_t>(kSlots, n_chunks);
     // buffers: s input, 4+s output, 8+s workspace, 12 small
     for (int s = 0; s < slots; ++s) {
@@ -488,7 +550,7 @@ int snappy_b200_compress_host_range(const void *in, uint64_t n_bytes, int mode, 
             e = cudaMemsetAsync(d_bytes, 0, 16, st);
         if (e == cudaSuccess)
             e = compress_chunk(static_cast<const uint8_t *>(g_ctx.buf[0 + s]), len, j == 0 ? varint_value : 0, mode,
-                               static_cast<uint8_t *>(g_ctx.buf[4 + s]), out_cap_chunk, d_bytes, d_status,
+                               framed, identifier && j == 0, static_cast<uint8_t *>(g_ctx.buf[4 + s]), out_cap_chunk, d_bytes, d_status,
                                g_ctx.buf[8 + s], st);
         if (e == cudaSuccess)
             e = cudaEventRecord(ev_run[s], st);
@@ -542,6 +604,66 @@ int snappy_b200_compress_host_range(const void *in, uint64_t n_bytes, int mode, 
     }
     *out_bytes = off;
     return SNAPPY_B200_OK;
+}
+
+extern "C" {
+
+int snappy_b200_compress_host_range(const void *in, uint64_t n_bytes, int mode, void *out, uint64_t out_capacity,
+                                    uint64_t *out_bytes, uint64_t *block_offsets, uint64_t varint_value)
+{
+    clear_error();
+    if (!out_bytes || (n_bytes && (!in || !out)))
+        return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
+    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
+        return fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
+    *out_bytes = 0;
+    if (n_bytes == 0)
+        return SNAPPY_B200_OK; // reference: an empty input gives an empty stream
+    if (env_devices() > 1 && n_bytes >= kMultiMin)
+        return snappy_b200_compress_host_multi_range(in, n_bytes, mode, out, out_capacity, out_bytes, block_offsets,
+                                                     env_devices(), varint_value);
+    return compress_host_chunks(in, n_bytes, mode, false, false, out, out_capacity, out_bytes, block_offsets,
+                                varint_value);
+}
+
+} // extern "C"
+
+namespace sb200 {
+// One range of a longer input as framed chunks, for callers that stream (the FILE* layer): n_bytes must be whole
+// 64 KiB blocks except for the last range; `identifier`: the range opens the stream.
+int frame_compress_host_range(const void *in, uint64_t n_bytes, int mode, void *out, uint64_t out_capacity,
+                              uint64_t *out_bytes, bool identifier)
+{
+    if (!out_bytes || !out || (n_bytes && !in))
+        return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
+    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
+        return fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
+    *out_bytes = 0;
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev < 1) { // no CPU path, also for the empty input
+        (void)cudaGetLastError();
+        return fail_msg(SNAPPY_B200_ERR_CUDA, "no CUDA device");
+    }
+    if (n_bytes == 0) {
+        if (!identifier)
+            return SNAPPY_B200_OK;
+        if (out_capacity < sizeof kStreamId)
+            return fail_msg(SNAPPY_B200_ERR_CAPACITY, "output buffer too small for the stream identifier");
+        memcpy(out, kStreamId, sizeof kStreamId);
+        *out_bytes = sizeof kStreamId;
+        return SNAPPY_B200_OK;
+    }
+    return compress_host_chunks(in, n_bytes, mode, true, identifier, out, out_capacity, out_bytes, nullptr, 0);
+}
+} // namespace sb200
+
+extern "C" {
+
+int snappy_b200_frame_compress_host(const void *in, uint64_t n_bytes, int mode, void *out, uint64_t out_capacity,
+                                    uint64_t *out_bytes)
+{
+    clear_error();
+    return frame_compress_host_range(in, n_bytes, mode, out, out_capacity, out_bytes, true);
 }
 
 int snappy_b200_uncompressed_length(const void *stream, uint64_t stream_bytes, uint64_t *n_bytes)
@@ -929,6 +1051,115 @@ int snappy_b200_decompress_host_indexed(const void *stream, uint64_t stream_byte
     clear_error();
     return decompress_host_general(stream, stream_bytes, out, out_bytes); // (all arguments were checked above)
 }
+
+// ---- framed streams: the chunk headers are walked on the host (the framing is the block index: no K0); the
+// stream goes up in pieces cut at chunk boundaries, growing like the indexed path's, and every piece is decoded
+// (k_frame_decode), checked (k_crc32c_chunks) and downloaded while the next one is in flight.
+int snappy_b200_frame_uncompressed_length(const void *stream, uint64_t stream_bytes, uint64_t *n_bytes)
+{
+    clear_error();
+    if (!n_bytes || (stream_bytes && !stream))
+        return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
+    return frame_walk(static_cast<const uint8_t *>(stream), stream_bytes, true, nullptr, n_bytes);
+}
+
+int snappy_b200_frame_decompress_host(const void *stream, uint64_t stream_bytes, void *out, uint64_t out_capacity,
+                                      uint64_t *out_bytes)
+{
+    clear_error();
+    return frame_decompress_buffer(stream, stream_bytes, out, out_capacity, out_bytes, true);
+}
+
+} // extern "C"
+
+namespace sb200 {
+// A whole framed stream (opens_stream) or, for the FILE* layer, a run of whole chunks from inside one.
+int frame_decompress_buffer(const void *stream, uint64_t stream_bytes, void *out, uint64_t out_capacity,
+                            uint64_t *out_bytes, bool opens_stream)
+{
+    if (!out_bytes || (stream_bytes && !stream))
+        return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
+    *out_bytes = 0;
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev < 1) { // no CPU path, also for streams without data
+        (void)cudaGetLastError();
+        return fail_msg(SNAPPY_B200_ERR_CUDA, "no CUDA device");
+    }
+    std::vector<FrameChunk> chunks;
+    uint64_t total = 0;
+    const int rc = frame_walk(static_cast<const uint8_t *>(stream), stream_bytes, opens_stream, &chunks, &total);
+    if (rc != SNAPPY_B200_OK)
+        return rc;
+    if (total > out_capacity)
+        return fail_msg(SNAPPY_B200_ERR_CAPACITY, "output buffer too small for the decompressed data");
+    if (total == 0) { // only empty data chunks (or none): each must be empty and carry the CRC of no bytes
+        for (const FrameChunk &c : chunks) // (a malformed chunk takes precedence over a checksum, as on the device)
+            if (c.in_len != 0)
+                return fail_msg(SNAPPY_B200_ERR_CORRUPT, "framed stream: an empty chunk with a non-empty body");
+        for (const FrameChunk &c : chunks)
+            if (c.crc != 0xa282ead8u) // mask(CRC-32C of no bytes = 0)
+                return fail_msg(SNAPPY_B200_ERR_CHECKSUM, "framed stream: a chunk's CRC-32C does not match its data");
+        return SNAPPY_B200_OK;
+    }
+    if (!out)
+        return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
+    HostCtx &g_ctx = current_ctx();
+    std::lock_guard<std::mutex> lock(g_ctx.mu);
+    CU(g_ctx.init(), "context init");
+    const uint64_t nc = chunks.size();
+    CU(g_ctx.need(0, stream_bytes + 64), "cudaMalloc");
+    CU(g_ctx.need(1, total), "cudaMalloc");
+    CU(g_ctx.need(4, nc * sizeof(FrameChunk)), "cudaMalloc");
+    CU(g_ctx.need(6, 256), "cudaMalloc");
+    uint8_t *d_stream = static_cast<uint8_t *>(g_ctx.buf[0]);
+    uint8_t *d_out = static_cast<uint8_t *>(g_ctx.buf[1]);
+    FrameChunk *d_chunks = static_cast<FrameChunk *>(g_ctx.buf[4]);
+    uint32_t *d_status = static_cast<uint32_t *>(g_ctx.buf[6]);
+    const uint8_t *src = static_cast<const uint8_t *>(stream);
+    uint8_t *dst = static_cast<uint8_t *>(out);
+    CU(cudaMemsetAsync(d_status, 0, 4, g_ctx.s_up), "memset");
+    CU(cudaMemcpyAsync(d_chunks, chunks.data(), nc * sizeof(FrameChunk), cudaMemcpyHostToDevice, g_ctx.s_up),
+       "H2D copy");
+    uint64_t launches = 0;
+    const uint64_t piece = kUploadPiece;
+    uint64_t c0 = 0, lo = 0, want = std::max<uint64_t>(piece / 8, 1 << 20);
+    int k = 0;
+    while (c0 < nc) {
+        // chunks [c0, c1): about `want` stream bytes; the last piece takes the rest of the stream
+        uint64_t c1 = c0 + 1;
+        while (c1 < nc && chunks[c1].in_off + chunks[c1].in_len - lo <= want)
+            ++c1;
+        const uint64_t hi = c1 == nc ? stream_bytes : chunks[c1 - 1].in_off + chunks[c1 - 1].in_len;
+        cudaEvent_t ev_up = g_ctx.ev[k & 7], ev_dec = g_ctx.ev[8 + (k & 7)];
+        CU(cudaMemcpyAsync(d_stream + lo, src + lo, hi - lo, cudaMemcpyHostToDevice, g_ctx.s_up), "H2D copy");
+        CU(cudaEventRecord(ev_up, g_ctx.s_up), "event record");
+        CU(cudaStreamWaitEvent(g_ctx.s_dec, ev_up, 0), "stream wait");
+        CU(launch_frame_decode(d_stream, stream_bytes, d_chunks + c0, c1 - c0, d_out, d_status, g_ctx.s_dec, &launches),
+           "decode launch");
+        CU(launch_frame_check(d_out, d_chunks + c0, c1 - c0, d_status, g_ctx.s_dec, &launches), "checksum launch");
+        CU(cudaEventRecord(ev_dec, g_ctx.s_dec), "event record");
+        CU(cudaStreamWaitEvent(g_ctx.s_down, ev_dec, 0), "stream wait");
+        const uint64_t out_lo = chunks[c0].out_off, out_hi = chunks[c1 - 1].out_off + chunks[c1 - 1].out_len;
+        CU(cudaMemcpyAsync(dst + out_lo, d_out + out_lo, out_hi - out_lo, cudaMemcpyDeviceToHost, g_ctx.s_down),
+           "D2H copy");
+        c0 = c1, lo = hi;
+        want = std::min(want * 2, piece);
+        ++k;
+    }
+    add_launches(launches);
+    CU(cudaStreamSynchronize(g_ctx.s_dec), "decode");
+    CU(peek_u32(reinterpret_cast<uint32_t *>(g_ctx.h_small + 1), d_status, 1, g_ctx.s_dec), "read-back");
+    CU(cudaStreamSynchronize(g_ctx.s_dec), "decode");
+    CU(cudaStreamSynchronize(g_ctx.s_down), "D2H copy");
+    const uint32_t status = (uint32_t)g_ctx.h_small[1];
+    if (status)
+        return status_error(status);
+    *out_bytes = total;
+    return SNAPPY_B200_OK;
+}
+} // namespace sb200
+
+extern "C" {
 
 // ---- device-level index-less decode (include/snappy_b200.h): the same piecewise loop on a
 // device-resident stream, with a library-owned second stream for the decode kernels.

@@ -25,8 +25,8 @@ int cuda_fail_msg(cudaError_t e, const char *what);
 int status_error(uint32_t st);
 void clear_error();
 void add_launches(uint64_t n);
-size_t compress_workspace_bytes_internal(uint64_t n_bytes);
-cudaError_t compress_chunk(const uint8_t *, uint64_t, uint64_t, int, uint8_t *, uint64_t, uint64_t *, uint32_t *, void *,
+size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed);
+cudaError_t compress_chunk(const uint8_t *, uint64_t, uint64_t, int, bool, bool, uint8_t *, uint64_t, uint64_t *, uint32_t *, void *,
                            cudaStream_t);
 const uint64_t *compress_chunk_offsets(void *, uint64_t);
 size_t index_workspace_bytes(uint64_t);
@@ -181,7 +181,7 @@ int snappy_b200_compress_host_multi_range(const void *in, uint64_t n_bytes, int 
         W(a.init(), "arena init");
         W(a.need(0, 2 * chunk), "cudaMalloc");                                            // two input slots
         W(a.need(1, max_compressed(hi - lo) + 32 * n_chunks + 64), "cudaMalloc");        // all compressed chunks
-        W(a.need(2, compress_workspace_bytes_internal(chunk)), "cudaMalloc");
+        W(a.need(2, compress_workspace_bytes_internal(chunk, false)), "cudaMalloc");
         W(a.need(3, 256), "cudaMalloc");
         uint8_t *d_in = static_cast<uint8_t *>(a.buf[0]);
         uint8_t *d_out = static_cast<uint8_t *>(a.buf[1]);
@@ -192,7 +192,7 @@ int snappy_b200_compress_host_multi_range(const void *in, uint64_t n_bytes, int 
             uint8_t *slot = d_in + (c & 1) * chunk;
             W(cudaMemcpyAsync(slot, src + clo, len, cudaMemcpyHostToDevice, a.st), "H2D copy");
             W(cudaMemsetAsync(d_small, 0, 16, a.st), "memset");
-            W(compress_chunk(slot, len, (g == 0 && c == 0) ? varint_value : 0, mode, d_out + doff, max_compressed(len), d_small,
+            W(compress_chunk(slot, len, (g == 0 && c == 0) ? varint_value : 0, mode, false, false, d_out + doff, max_compressed(len), d_small,
                              reinterpret_cast<uint32_t *>(d_small + 1), a.buf[2], a.st),
               "compress launch");
             W(cudaMemcpyAsync(a.h_small, d_small, 16, cudaMemcpyDeviceToHost, a.st), "read-back");
