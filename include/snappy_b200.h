@@ -60,7 +60,7 @@ extern "C" {
 #define SNAPPY_B200_ST_CAPACITY 1u
 #define SNAPPY_B200_ST_CORRUPT 2u
 #define SNAPPY_B200_ST_FRAMING 4u
-#define SNAPPY_B200_ST_UNRESOLVED 8u /* the element chain did not resolve within the relaxation rounds run */
+#define SNAPPY_B200_ST_UNRESOLVED 8u /* async decode only: the element chain did not resolve within max_rounds */
 #define SNAPPY_B200_ST_CHECKSUM 16u  /* framed stream: a chunk's CRC-32C does not match (CORRUPT takes precedence) */
 
 /* Message of the last failing call on this thread (never NULL). */
@@ -123,7 +123,11 @@ int snappy_b200_decode_segments_device(const uint8_t *d_stream, uint64_t stream_
  * runs on a library-owned second stream that is joined back into `stream` before the call
  * returns).  d_block_offsets [n_blocks+1] (optional) is filled as a by-product.
  * Workspace: snappy_b200_decompress_workspace_bytes.  Synchronises `stream` between K0
- * rounds; the last decode is only enqueued.                                                */
+ * rounds; the last decode is only enqueued.  K0 here (and in snappy_b200_index_device, the
+ * host-buffer and FILE* calls) runs rounds until the element chain is resolved, which every
+ * valid stream is after at most one round per 8 KiB of stream (adversarial input needs about
+ * that many; ordinary streams a few dozen): these calls never give SNAPPY_B200_ST_UNRESOLVED,
+ * which only snappy_b200_decompress_device_async reports.                                  */
 size_t snappy_b200_decompress_workspace_bytes(uint64_t stream_bytes, uint64_t total_out);
 int snappy_b200_decompress_device(const uint8_t *d_stream, uint64_t stream_bytes, uint64_t body_offset,
                                   uint64_t total_out, uint8_t *d_out, uint64_t *d_block_offsets,

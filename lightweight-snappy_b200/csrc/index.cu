@@ -926,11 +926,15 @@ const uint64_t *index_total(void *d_ws, uint64_t stream_bytes) { return carve(d_
 // The relaxation rounds end on the device: every round reads the "changed" flag of the round before and
 // returns at once when it is clear, so a batch of rounds can be enqueued blind.
 //   fixed_rounds == 0  adaptive: batches of 16, 48, 64, ... rounds, the flags read back after each batch
-//                      (synchronises the stream); gives up with ST_UNRESOLVED after kMaxRounds.
+//                      (synchronises the stream), until a round changes nothing.  A chain over ngroup groups is
+//                      resolved after at most ngroup rounds and one more shows that nothing moves, so every
+//                      valid stream converges within max_rounds = ngroup + 2 + one batch; an adversarial one
+//                      (tests/k0gen.py: every speculative walk misses the chain) needs about ngroup rounds, which
+//                      costs time linear in the stream, the order of the sequential walk of the general decoder.
+//                      ST_UNRESOLVED from this mode can only mean a bug in K0.
 //   fixed_rounds  > 0  asynchronous: exactly one batch of min(fixed_rounds, 64) rounds, no read-back, no
 //                      synchronisation (graph-capturable); ST_UNRESOLVED if its last round still moved.
 constexpr uint32_t kMaxBatch = 64;
-constexpr uint64_t kMaxRounds = 1u << 14; // an adversarial stream may need one round per group: bounded instead
 
 cudaError_t run_index(const uint8_t *d_stream, uint64_t stream_bytes, uint64_t body_offset, uint64_t total_out,
                       uint64_t *d_block_offsets, uint32_t *d_status, void *d_ws, cudaStream_t st, uint64_t *launches,
@@ -962,7 +966,7 @@ cudaError_t run_index(const uint8_t *d_stream, uint64_t stream_bytes, uint64_t b
                                         !open_end && getenv("SNAPPY_B200_K0_NO_RUNUP") == nullptr &&
                                             stream_bytes / 4 >= total_out / 5);
     *launches += 2;
-    const uint64_t max_rounds = std::min<uint64_t>(ngroup + 2 + kMaxBatch, kMaxRounds);
+    const uint64_t max_rounds = ngroup + 2 + kMaxBatch;
     const uint32_t *unresolved = nullptr; // flag of the last round run, when nothing proves convergence
     uint32_t batch = fixed_rounds ? std::min<uint32_t>(fixed_rounds, kMaxBatch) : 16;
     // a chain over ngroup groups is resolved after at most ngroup rounds (one more shows that nothing moves):
