@@ -18,11 +18,11 @@
 // not write compressed bytes: it leaves one 8-byte record per copy {position, offset,
 // length, literal run before it}.
 //
-// Hash-mode table: u16 position + u8 key fingerprint per slot, in two arrays (8 + 4 KiB, so 18
-// blocks fit in one SM's shared memory).  The fingerprint is bits 19..12 of key*0x1e35a7bd --
-// together with the 12-bit slot index it pins 20 of the 32 bits of an injective function of
-// the key, so the "does the candidate's 4 bytes equal mine" test of the reference
-// (found_match, :259-265) is almost always answered from shared memory; lanes whose
+// Hash-mode table: u16 position + u8 key fingerprint per slot, in two arrays (8 KiB in global
+// memory, 4 KiB in shared memory, see k_parse_hash_global).  The fingerprint is bits 19..12 of
+// key*0x1e35a7bd -- together with the 12-bit slot index it pins 20 of the 32 bits of an
+// injective function of the key, so the "does the candidate's 4 bytes equal mine" test of the
+// reference (found_match, :259-265) is almost always answered from shared memory; lanes whose
 // fingerprint matches confirm against the candidate bytes, all at once, and compare the next
 // four bytes in the same fetch (most matches end there, which saves the separate extension
 // round trip).  The reference's zero-filled table ("candidate = position 0") becomes
@@ -38,7 +38,6 @@
 // prefix-summed and written in parallel into the block's scratch slot; long literals are
 // copied by the whole CTA with 16-byte stores.
 #include <algorithm>
-#include <cstdlib>
 
 #include <mutex>
 #include <type_traits>
@@ -145,7 +144,8 @@ template <int LOG_SLOTS, bool GLOBAL = false> struct ExactTable {
 };
 
 // ------------------------------------------------------------------------------- the parse
-// MODE 0 = hash table (LOG_SLOTS ignored: the table has up to 4096 u32 entries)
+// MODE 0 = hash table (LOG_SLOTS ignored: up to 4096 u16 positions at smem_raw, one u8 fingerprint per
+//          slot at fp_mem)
 // MODE 1 = exact dictionary with 2^LOG_SLOTS u16 slots; a block whose dictionary would grow
 //          past 3/4 of the table gives up (nrec[blk] = kAbortMark) unless FINAL.
 // smem_raw: the table memory (shared, or global when GLOBAL).
@@ -168,8 +168,8 @@ __device__ __forceinline__ void parse_block(const uint8_t *__restrict__ in, uint
     constexpr uint32_t C = MODE == 0 ? 1 : 2;
     constexpr uint32_t D = MODE == 0 ? 0 : 1;
 
-    uint16_t *hpos = reinterpret_cast<uint16_t *>(smem_raw);   // hash mode: candidate position per slot
-    uint8_t *hfp = fp_mem ? fp_mem : smem_raw + 2 * SNAPPY_B200_HTABLE_SIZE; // hash mode: key fingerprint per slot
+    uint16_t *hpos = reinterpret_cast<uint16_t *>(smem_raw); // hash mode: candidate position per slot
+    uint8_t *hfp = fp_mem;                                    // hash mode: key fingerprint per slot
     ExactTable<LOG_SLOTS, GLOBAL> et{reinterpret_cast<typename ExactTable<LOG_SLOTS, GLOBAL>::Entry *>(smem_raw)};
     uint32_t shift = 20;
     uint32_t n_keys = 0; // exact mode: dictionary population (warp-uniform)
@@ -526,15 +526,16 @@ __device__ __forceinline__ void parse_block(const uint8_t *__restrict__ in, uint
         nrec[blk] = nh;
 }
 
-template <int MODE, int LOG_SLOTS, bool FINAL>
+// The big exact tiers with the table in shared memory, one CTA per block: only the blocks an earlier tier gave up on.
+template <int LOG_SLOTS, bool FINAL>
 __global__ void __launch_bounds__(32) k_parse(const uint8_t *__restrict__ in, uint64_t n_bytes,
-                                              uint2 *__restrict__ recs, uint32_t *__restrict__ nrec, int only_marked)
+                                              uint2 *__restrict__ recs, uint32_t *__restrict__ nrec)
 {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     const uint64_t blk = blockIdx.x;
-    if (only_marked && nrec[blk] != kAbortMark)
+    if (nrec[blk] != kAbortMark)
         return;
-    parse_block<MODE, LOG_SLOTS, FINAL>(in, n_bytes, recs, nrec, blk, smem_raw);
+    parse_block<1, LOG_SLOTS, FINAL>(in, n_bytes, recs, nrec, blk, smem_raw);
 }
 
 // The big exact tier: 2^16 slots (128 KiB) per chain do not fit many times into shared memory
@@ -568,7 +569,7 @@ __global__ void __launch_bounds__(32) k_parse_exact_global(const uint8_t *__rest
 // 32 per SM, each with its own tables, taking blocks from a counter.  With nothing in shared
 // memory the SM's whole 256 KB is L1, which keeps the hot part of the tables close, and 32
 // latency-bound chains per SM beat the 17-18 that 12 KiB shared-memory tables allow (measured:
-// 16.0 -> 14.0 ms per GiB of the mixed corpus; the k_parse<0> kernel is the shared-memory version).
+// 16.0 -> 14.0 ms per GiB of the mixed corpus, DESIGN.md §4).
 __global__ void __launch_bounds__(32) k_parse_hash_global(const uint8_t *__restrict__ in, uint64_t n_bytes,
                                                           uint64_t n_blocks, uint2 *__restrict__ recs,
                                                           uint32_t *__restrict__ nrec, uint8_t *__restrict__ tables,
@@ -774,16 +775,11 @@ cudaError_t launch_compress(const uint8_t *d_in, uint64_t n_bytes, int mode, uin
     const uint64_t chains = std::min<uint64_t>(nb, (uint64_t)n_sm * 32); // one-warp CTAs: 32 per SM
     const uint64_t area = nb * (uint64_t)kSlot - 256;
     uint32_t *counters = reinterpret_cast<uint32_t *>(d_scratch + area);
-    // the measured alternative (DESIGN.md 6); read per call: the test suite flips it between calls
-    const bool smem_tables = getenv("SNAPPY_B200_SMEM_TABLES") != nullptr;
-    cudaError_t e = smem_tables ? cudaSuccess : cudaMemsetAsync(counters, 0, 16, st);
+    cudaError_t e = cudaMemsetAsync(counters, 0, 16, st);
     if (e != cudaSuccess)
         return e;
     if (mode == SNAPPY_B200_MODE_HASH) {
-        if (smem_tables)
-            k_parse<0, 12, true><<<grid, cta, 4096 * 3, st>>>(d_in, n_bytes, d_recs, d_nrec, 0);
-        else
-            k_parse_hash_global<<<(unsigned)chains, cta, 0, st>>>(d_in, n_bytes, nb, d_recs, d_nrec, d_scratch, counters);
+        k_parse_hash_global<<<(unsigned)chains, cta, 0, st>>>(d_in, n_bytes, nb, d_recs, d_nrec, d_scratch, counters);
         *launches += 1;
     } else {
         // exact mode: 8 Ki slots (16 KiB), then 64 Ki slots (128 KiB) for the blocks that outgrow them
@@ -791,26 +787,22 @@ cudaError_t launch_compress(const uint8_t *d_in, uint64_t n_bytes, int mode, uin
         // (the opt-in to > 48 KiB of dynamic shared memory is per device: once per device, thread-safe)
         static std::once_flag attr_once[64];
         std::call_once(attr_once[dev & 63], [&] {
-            e = cudaFuncSetAttribute(k_parse<1, 15, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (1 << 15) * 2);
+            e = cudaFuncSetAttribute(k_parse<15, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (1 << 15) * 2);
             if (e == cudaSuccess)
-                e = cudaFuncSetAttribute(k_parse<1, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (1 << 16) * 2);
+                e = cudaFuncSetAttribute(k_parse<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (1 << 16) * 2);
         });
         if (e != cudaSuccess)
             return e;
-        if (smem_tables)
-            k_parse<1, 13, false><<<grid, cta, (1 << 13) * 2, st>>>(d_in, n_bytes, d_recs, d_nrec, 0);
-        else
-            k_parse_exact_global<13, false><<<(unsigned)chains, cta, 0, st>>>(d_in, n_bytes, nb, d_recs, d_nrec,
-                                                                              d_scratch, counters + 1, 0);
+        k_parse_exact_global<13, false><<<(unsigned)chains, cta, 0, st>>>(d_in, n_bytes, nb, d_recs, d_nrec, d_scratch,
+                                                                          counters + 1, 0);
         const uint64_t n_big = std::min<uint64_t>(area / ((uint64_t)4 << kGlobalTierLog), chains);
-        if (n_big >= 1 && !smem_tables) {
+        if (n_big >= 1) {
             k_parse_exact_global<kGlobalTierLog, true><<<(unsigned)n_big, cta, 0, st>>>(d_in, n_bytes, nb, d_recs, d_nrec,
                                                                                      d_scratch, counters + 2, 1);
             *launches += 2;
-        } else { // a single block (or the A/B switch): the big tiers in shared memory
-            k_parse<1, 15, false><<<grid, cta, (1 << 15) * 2, st>>>(d_in, n_bytes, d_recs, d_nrec, 1);
-            k_parse<1, 16, true><<<grid, cta, (1 << 16) * 2, st>>>(d_in, n_bytes, d_recs, d_nrec, 1);
+        } else { // 1 to 3 blocks: the output slots cannot hold one 256 KiB table, so the big tiers go to shared memory
+            k_parse<15, false><<<grid, cta, (1 << 15) * 2, st>>>(d_in, n_bytes, d_recs, d_nrec);
+            k_parse<16, true><<<grid, cta, (1 << 16) * 2, st>>>(d_in, n_bytes, d_recs, d_nrec);
             *launches += 3;
         }
     }

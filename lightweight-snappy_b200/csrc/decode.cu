@@ -190,12 +190,6 @@ struct SegSmem {
     uint32_t bm[kRunBytes / 32 + 4]; // element starts inside the current run, one bit per output byte
 };
 
-// How produce_run resolves a copy whose source byte is produced by the same round.
-enum class Produce {
-    kShuffle, // pointer doubling over the lanes of the round (the product)
-    kFollow,  // each lane follows its chain back through the table (SNAPPY_B200_DECODE_PRODUCE=follow, A/B)
-};
-
 // Bit 31 of a source position: the byte is in the stream (relative to `in`), not in the output (relative
 // to the block's `out`, always below 65536).  A literal's stream position is below 2 * 65536 + 256.
 constexpr uint32_t kFromStream = 0x80000000u;
@@ -203,111 +197,66 @@ constexpr uint32_t kFromStream = 0x80000000u;
 // Table entry of an element that starts at window-relative output byte `start` (after it: `len` bytes,
 // offset `info` for a copy, stream position `info` of the first literal byte):
 //   x = start, y = offset (0: literal) | (floor(2^15/offset)+1) << 16 when the copy overlaps itself,
-//   kShuffle: z = source position of window byte 0, so that window byte k comes from position z + k (32-bit
-//             wrap-around), kFromStream set for a literal;
-//   kFollow:  (z,w) = pointer p such that window byte k is p[k] -- the stream for a literal, out + op - offset
-//             for a copy.
+//   z = source position of window byte 0, so that window byte k comes from position z + k (32-bit wrap-around),
+//   kFromStream set for a literal; w is unused.
 // A special element (one-element path) has y = 0xffffffff and z = the stream position `pos` of its tag.
-template <Produce P>
-__device__ __forceinline__ uint4 seg_entry(const uint8_t *in, uint8_t *out, uint32_t op, uint32_t start,
-                                           const Header &h, uint32_t len, uint32_t pos, bool special)
+__device__ __forceinline__ uint4 seg_entry(uint32_t op, uint32_t start, const Header &h, uint32_t len, uint32_t pos,
+                                           bool special)
 {
     if (special)
         return make_uint4(start, 0xffffffffu, pos, 0u);
     const uint32_t off = h.is_lit ? 0u : h.info; // <= 65535 (copy-4 is special)
     const uint32_t y = off | (off != 0 && off < len ? (32768u / off + 1u) << 16 : 0u);
-    if (P != Produce::kFollow)
-        return make_uint4(start, y, h.is_lit ? h.info - start + kFromStream : op - off, 0u);
-    const uint8_t *p = h.is_lit ? in + h.info - start : out + op - off;
-    const uint64_t pa = reinterpret_cast<uint64_t>(p);
-    return make_uint4(start, y, (uint32_t)pa, (uint32_t)(pa >> 32));
+    return make_uint4(start, y, h.is_lit ? h.info - start + kFromStream : op - off, 0u);
 }
 
 // Produces the output bytes [k_lo, k_hi) (window-relative) of the elements e_lo.. of the table;
-// `bm` holds their starts relative to k_lo.  Same per-byte rule as produce() above.
+// `bm` holds their starts relative to k_lo.  Same per-byte rule as produce() above, but a source byte produced
+// by the same round is resolved by pointer doubling instead of following the chain back.
 //
-// kShuffle: the lane of byte k = c + lane looks its element up once.  A literal, or a copy whose source
-// byte s = kk - offset lies before the round (s < c), is a root and knows the position it reads; any other
-// lane copies lane s - c < lane, its parent.  Five pointer-doubling shuffles take every lane to its root
-// (a chain inside a round has fewer than 32 links), one more fetches the root's position, and every lane
-// does exactly one load.  Rounds in which no lane has a parent skip the shuffles.  (Measured, B200, 1 GiB
-// per class: a doubling loop that ends on a ballot once every parent is a root lost on low-entropy data,
-// 3.83 against 3.64 ms; five shuffles in every round lost on text, 6.10 against 5.88 ms.)
-// Following a chain back one link computes, for k' = kk - offset, the same element look-up and kk' that
-// lane k' - c computes for itself, so both variants read the same byte.
-template <Produce P>
+// The lane of byte k = c + lane looks its element up once.  A literal, or a copy whose source byte
+// s = kk - offset lies before the round (s < c), is a root and knows the position it reads; any other lane
+// copies lane s - c < lane, its parent.  Five pointer-doubling shuffles take every lane to its root (a chain
+// inside a round has fewer than 32 links), one more fetches the root's position, and every lane does exactly
+// one load.  Rounds in which no lane has a parent skip the shuffles.  (Measured, B200, 1 GiB per class: a
+// doubling loop that ends on a ballot once every parent is a root lost on low-entropy data, 3.83 against
+// 3.64 ms; five shuffles in every round lost on text, 6.10 against 5.88 ms; following each chain back through
+// the table, as produce() does, lost too, DESIGN.md §6.)
 __device__ __forceinline__ void produce_run(const uint8_t *__restrict__ in, uint8_t *out, uint32_t op, uint32_t k_lo,
                                             uint32_t k_hi, uint32_t e_lo, const SegSmem &sm, uint32_t lane)
 {
     const unsigned le_mask = 0xffffffffu >> (31u - lane);
     uint32_t before = e_lo; // table index of the first element that starts in this round, if any does
     uint8_t *o = out + op + k_lo + lane;
-    if constexpr (P != Produce::kFollow) {
-        for (uint32_t c = k_lo; c < k_hi; c += 32, o += 32) {
-            const unsigned B = sm.bm[(c - k_lo) >> 5];
-            // every lane's look-up is a valid table entry (the element at or before it), also past k_hi
-            const uint4 e = sm.elems[before + __popc(B & le_mask) - 1u];
-            const uint32_t off = e.y & 0xffffu, inv = e.y >> 16;
-            uint32_t kk = c + lane;
-            if (inv) { // write_copy :273-280: byte i comes from i mod offset when the copy overlaps itself
-                const uint32_t i = kk - e.x;
-                kk = e.x + i - off * ((i * inv) >> 15);
-            }
-            uint32_t src = e.z + kk;
-            // produced by this very round: the parent is a lower lane (a lane past k_hi has no children)
-            uint32_t parent = off != 0 && kk >= c + off ? kk - off - c : lane;
-            if (__any_sync(kFull, parent != lane)) {
+    for (uint32_t c = k_lo; c < k_hi; c += 32, o += 32) {
+        const unsigned B = sm.bm[(c - k_lo) >> 5];
+        // every lane's look-up is a valid table entry (the element at or before it), also past k_hi
+        const uint4 e = sm.elems[before + __popc(B & le_mask) - 1u];
+        const uint32_t off = e.y & 0xffffu, inv = e.y >> 16;
+        uint32_t kk = c + lane;
+        if (inv) { // write_copy :273-280: byte i comes from i mod offset when the copy overlaps itself
+            const uint32_t i = kk - e.x;
+            kk = e.x + i - off * ((i * inv) >> 15);
+        }
+        uint32_t src = e.z + kk;
+        // produced by this very round: the parent is a lower lane (a lane past k_hi has no children)
+        uint32_t parent = off != 0 && kk >= c + off ? kk - off - c : lane;
+        if (__any_sync(kFull, parent != lane)) {
 #pragma unroll
-                for (int d = 0; d < 5; ++d)
-                    parent = __shfl_sync(kFull, parent, parent);
-                src = __shfl_sync(kFull, src, parent);
-            }
-            if (c + lane < k_hi) {
-                const uint8_t *base = (src & kFromStream) ? in : out;
-                *o = base[src & ~kFromStream];
-            }
-            before += __popc(B);
-            __syncwarp(); // the next round may read what this one wrote
+            for (int d = 0; d < 5; ++d)
+                parent = __shfl_sync(kFull, parent, parent);
+            src = __shfl_sync(kFull, src, parent);
         }
-    } else {
-        for (uint32_t c = k_lo; c < k_hi; c += 32, o += 32) {
-            const unsigned B = sm.bm[(c - k_lo) >> 5];
-            uint32_t k = c + lane;
-            bool pending = k < k_hi;
-            uint32_t val = 0;
-            uint32_t r = before + __popc(B & le_mask) - 1u;
-            for (;;) {
-                if (pending) {
-                    const uint4 e = sm.elems[r];
-                    const uint32_t off = e.y & 0xffffu, inv = e.y >> 16;
-                    uint32_t kk = k;
-                    if (inv) { // write_copy :273-280: byte i comes from i mod offset when the copy overlaps itself
-                        const uint32_t i = k - e.x;
-                        kk = e.x + i - off * ((i * inv) >> 15);
-                    }
-                    if (off == 0 || kk < c + off) {
-                        // a literal, or a copy whose source was written by an earlier step / round
-                        const uint8_t *p = reinterpret_cast<const uint8_t *>(((uint64_t)e.w << 32) | e.z);
-                        val = p[kk];
-                        pending = false;
-                    } else {
-                        k = kk - off; // produced by this very round: follow it back
-                        r = before + __popc(B & (0xffffffffu >> (31u - (k - c)))) - 1u;
-                    }
-                }
-                if (!__any_sync(kFull, pending))
-                    break;
-            }
-            if (c + lane < k_hi)
-                *o = (uint8_t)val;
-            before += __popc(B);
-            __syncwarp(); // the next round may read what this one wrote
+        if (c + lane < k_hi) {
+            const uint8_t *base = (src & kFromStream) ? in : out;
+            *o = base[src & ~kFromStream];
         }
+        before += __popc(B);
+        __syncwarp(); // the next round may read what this one wrote
     }
 }
 
-template <int MINB, Produce P>
-__global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restrict__ stream, uint64_t body_offset,
+__global__ void __launch_bounds__(64, 20) k_decode_seg(const uint8_t *__restrict__ stream, uint64_t body_offset,
                                                          const uint64_t *__restrict__ offsets,
                                                          const uint4 *__restrict__ starts, uint64_t total_out,
                                                          uint8_t *out_base, uint32_t *__restrict__ status,
@@ -434,9 +383,9 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
         const unsigned S = __ballot_sync(kFull, sp0 || sp1);
         // ---- the table
         if (has0)
-            sm.elems[rank] = seg_entry<P>(in, out, op, start0, h0, len0, pos0, sp0);
+            sm.elems[rank] = seg_entry(op, start0, h0, len0, pos0, sp0);
         if (has1)
-            sm.elems[rank + 1] = seg_entry<P>(in, out, op, start1, h1, len1, pos1, sp1);
+            sm.elems[rank + 1] = seg_entry(op, start1, h1, len1, pos1, sp1);
         if (S == 0) {
             // ---- the ordinary segment: one run
             const uint32_t words = (T + 31) >> 5;
@@ -448,7 +397,7 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
             if (has1)
                 atomicOr(&sm.bm[start1 >> 5], 1u << (start1 & 31u));
             __syncwarp(); // also: stores of earlier steps are visible to every lane from here
-            produce_run<P>(in, out, op, 0, T, 0, sm, lane);
+            produce_run(in, out, op, 0, T, 0, sm, lane);
         } else {
             // ---- runs of ordinary elements between the special ones (long literals, copy-4, ...)
             __syncwarp();
@@ -474,7 +423,7 @@ __global__ void __launch_bounds__(64, MINB) k_decode_seg(const uint8_t *__restri
                     if (has1 && rank + 1 >= e_lo && rank + 1 < e_hi)
                         atomicOr(&sm.bm[(start1 - k_lo) >> 5], 1u << ((start1 - k_lo) & 31u));
                     __syncwarp();
-                    produce_run<P>(in, out, op, k_lo, k_hi, e_lo, sm, lane);
+                    produce_run(in, out, op, k_lo, k_hi, e_lo, sm, lane);
                 }
                 if (e_hi < ne) {
                     uint32_t ip = sm.elems[e_hi].z, o2 = op + k_hi;
@@ -815,26 +764,16 @@ cudaError_t launch_decode_seg(const uint8_t *d_stream, uint64_t body_offset, con
         return e;
     // The order array lives in the memory of K0's per-segment output offsets, which this decoder does not need
     // (8 bytes per 128 stream bytes; a 64 KiB block is at least 2 KiB of stream, so it always fits).
-    static const bool in_order = getenv("SNAPPY_B200_DECODE_IN_ORDER") != nullptr; // A/B: blocks in stream order
     uint32_t *d_order = nullptr;
-    if (!in_order && d_outoff && n_blocks > 1) {
+    if (d_outoff && n_blocks > 1) {
         d_order = reinterpret_cast<uint32_t *>(const_cast<uint64_t *>(d_outoff));
         k_block_order<<<1, 1024, 0, st>>>(d_offsets, n_blocks, d_status, d_order);
         *launches += 1;
     }
     // two blocks (warps) per CTA and a 48-register cap: 40 warps per SM instead of the 32 that one-warp
     // CTAs allow (measured: 64 registers / 32 warps 6.92, 48 / 40 6.72, 40 / 48 6.84 ms per GiB, K0 included)
-    static const char produce = [] { // A/B: SNAPPY_B200_DECODE_PRODUCE=follow selects the follow-back loop
-        const char *v = getenv("SNAPPY_B200_DECODE_PRODUCE");
-        return v ? v[0] : 's';
-    }();
-    const unsigned grid = (unsigned)((n_blocks + 1) / 2);
-    if (produce == 'f')
-        k_decode_seg<20, Produce::kFollow><<<grid, 64, 0, st>>>(d_stream, body_offset, d_offsets, d_starts, total_out,
+    k_decode_seg<<<(unsigned)((n_blocks + 1) / 2), 64, 0, st>>>(d_stream, body_offset, d_offsets, d_starts, total_out,
                                                                 d_out, d_status, n_blocks, blk_base, d_order);
-    else
-        k_decode_seg<20, Produce::kShuffle><<<grid, 64, 0, st>>>(d_stream, body_offset, d_offsets, d_starts, total_out,
-                                                                 d_out, d_status, n_blocks, blk_base, d_order);
     *launches += 1;
     return cudaGetLastError();
 }

@@ -1161,29 +1161,15 @@ int frame_decompress_buffer(const void *stream, uint64_t stream_bytes, void *out
 
 extern "C" {
 
-// ---- device-level index-less decode (include/snappy_b200.h): the same piecewise loop on a
+// ---- device-level index-less decode (include/snappy_b200.h): the piecewise loop of the host path on a
 // device-resident stream, with a library-owned second stream for the decode kernels.
 // A device-resident stream is decoded as ONE piece: K0 has about 2 ms of latency-bound fixed cost
 // per call (measured, profiles/), so splitting only pays when there is a transfer to hide.
-// Pieces of a device-resident stream: K0 of piece p+1 (load/store-unit bound) overlaps the block decode
-// of piece p (issue bound) on the second stream.  SNAPPY_B200_DEVICE_PIECES sets how many (default 1).
-static uint64_t device_piece_bytes(uint64_t stream_bytes)
-{
-    static const uint64_t pieces = [] {
-        const char *v = getenv("SNAPPY_B200_DEVICE_PIECES");
-        const long k = v ? atol(v) : 1;
-        return (uint64_t)(k < 1 ? 1 : (k > 64 ? 64 : k));
-    }();
-    const uint64_t piece = (stream_bytes + pieces - 1) / pieces;
-    return std::max<uint64_t>(std::max<uint64_t>(piece, std::min<uint64_t>(stream_bytes, 8u << 20)), 1);
-}
-
+// The workspace has room for two piece slots (K0 workspace + block offsets); one piece uses the first.
 size_t snappy_b200_decompress_workspace_bytes(uint64_t stream_bytes, uint64_t total_out)
 {
-    const uint64_t piece = device_piece_bytes(stream_bytes);
     const uint64_t nb = (total_out + kBlock - 1) / kBlock;
-    const size_t per_slot = align_up(index_workspace_bytes(piece_region_cap(stream_bytes, piece)), 256) +
-                            align_up((nb + 2) * 8, 256);
+    const size_t per_slot = align_up(index_workspace_bytes(stream_bytes), 256) + align_up((nb + 2) * 8, 256);
     return 2 * per_slot + 256;
 }
 
@@ -1204,9 +1190,8 @@ int snappy_b200_decompress_device(const uint8_t *d_stream, uint64_t stream_bytes
                                            : fail_msg(SNAPPY_B200_ERR_CORRUPT, "trailing bytes after an empty stream");
     std::lock_guard<std::mutex> lock(g_ctx.mu);
     CU(g_ctx.init(), "context init");
-    const uint64_t piece = device_piece_bytes(stream_bytes);
     const uint64_t nb = (total_out + kBlock - 1) / kBlock;
-    const size_t ws_slot = align_up(index_workspace_bytes(piece_region_cap(stream_bytes, piece)), 256);
+    const size_t ws_slot = align_up(index_workspace_bytes(stream_bytes), 256);
     const size_t off_slot = align_up((nb + 2) * 8, 256);
     uint8_t *w = static_cast<uint8_t *>(d_workspace);
     PieceResources r;
@@ -1220,13 +1205,9 @@ int snappy_b200_decompress_device(const uint8_t *d_stream, uint64_t stream_bytes
     r.s_dec = g_ctx.s_dec;
     r.h_small = g_ctx.h_small + 8;
     PieceHooks hooks; // nothing to wait for, nothing to download
-    std::vector<uint64_t> piece_end;
-    for (uint64_t at = 0; at < stream_bytes;) {
-        at = std::min<uint64_t>(stream_bytes, at + piece);
-        piece_end.push_back(at);
-    }
+    const std::vector<uint64_t> piece_end = {stream_bytes}; // one piece, the whole stream
     const int rc = decode_pieces(d_stream, stream_bytes, body_offset, total_out, d_out, d_block_offsets, d_status,
-                                 piece_end, piece_region_cap(stream_bytes, piece), r, hooks);
+                                 piece_end, stream_bytes, r, hooks);
     if (rc != SNAPPY_B200_OK)
         return rc;
     // join: work the caller enqueues next on `stream` sees the decoded output

@@ -26,12 +26,13 @@
 //                      128-byte walks do NOT merge by themselves: lanes re-walk different
 //                      segments in parallel here instead of one serial chase per group.)
 //                      The groups themselves are resolved by the same relaxation one level up
-//                      (k_group_scatter / k_group_apply, one kernel pair per round; group 0's
-//                      entry is known).  Keeping dead groups talking matters: when a
-//                      mis-speculated "long literal" wrongly kills a run of groups they all
-//                      come back in the round after it is corrected instead of one per round.
+//                      (k_group_scatter / k_group_apply in round 0, then one fused k_group_apply32
+//                      per round; group 0's entry is known).  Keeping dead groups talking
+//                      matters: when a mis-speculated "long literal" wrongly kills a run of
+//                      groups they all come back in the round after it is corrected instead of
+//                      one per round.
 //                      Runs of incompressible blocks are chains of maximal literals that can
-//                      only be found one from the other; k_group_scatter looks 24 of them ahead.
+//                      only be found one from the other; scatter_group looks 24 of them ahead.
 //                      An adversarial stream degrades to sequential but stays correct.
 //   C  (k_group_final) every live segment sums the output bytes of its elements and stores the
 //                      exact bit map of its element starts (for the segment-driven decoder)
@@ -42,7 +43,6 @@
 //                      reported as SNAPPY_B200_ST_FRAMING.
 #include <algorithm>
 #include <atomic>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -313,8 +313,7 @@ __global__ void __launch_bounds__(kGroupCta) k_group_init(const uint8_t *__restr
                                                           uint32_t *__restrict__ g_entry, uint64_t *__restrict__ g_exit,
                                                           uint64_t *__restrict__ g_vis,
                                                           unsigned long long *__restrict__ g_claim,
-                                                          uint8_t *__restrict__ entries, int getenv_runup,
-                                                          int literal_scan)
+                                                          uint8_t *__restrict__ entries, int literal_scan)
 {
     __shared__ GroupStage stage[kGroupCta / 32];
     const uint64_t g = blockIdx.x * (uint64_t)(kGroupCta / 32) + (threadIdx.x >> 5);
@@ -363,7 +362,7 @@ __global__ void __launch_bounds__(kGroupCta) k_group_init(const uint8_t *__restr
     }
     if (lit_end != kNone) {
         e0 = lit_end;
-    } else if (g > 0 && getenv_runup) {
+    } else if (g > 0) {
         const uint64_t g_lo = g * kGroupBytes, g_hi = min(g_lo + kGroupBytes, body_len);
         const uint64_t s_last = g * kGroup - 1;
         for (int back = 2; back >= 0; --back) {
@@ -463,11 +462,8 @@ __device__ __forceinline__ void scatter_group(const uint8_t *__restrict__ body, 
 __global__ void __launch_bounds__(128) k_group_scatter(const uint8_t *__restrict__ body, uint64_t body_len,
                                                        uint64_t ngroup, const uint32_t *__restrict__ g_entry,
                                                        const uint64_t *__restrict__ g_exit,
-                                                       unsigned long long *__restrict__ g_claim,
-                                                       const uint32_t *__restrict__ prev_changed)
+                                                       unsigned long long *__restrict__ g_claim)
 {
-    if (prev_changed && *prev_changed == 0)
-        return; // the round before changed nothing: the fixed point is reached, the rest of the batch is idle
     const uint64_t g = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     if (g >= ngroup)
         return;
@@ -601,7 +597,7 @@ __global__ void __launch_bounds__(kGroupCta) k_group_apply32(const uint8_t *__re
     // Fused: what this group tells the next round goes straight into the other claim buffer (the claims this
     // round read are in g_claim, which every group has just reset for the round after next): one kernel per
     // round instead of two.
-    if (claim_out && g < ngroup) {
+    if (g < ngroup) {
         __syncwarp(); // (lane 0's g_exit of a re-resolved group is visible to the lane that owns the group)
         scatter_group(body, body_len, ngroup, g, *reinterpret_cast<volatile uint32_t *>(g_entry + g),
                       *reinterpret_cast<volatile uint64_t *>(g_exit + g), claim_out);
@@ -961,10 +957,9 @@ cudaError_t run_index(const uint8_t *d_stream, uint64_t stream_bytes, uint64_t b
     const unsigned wgrid32 = (unsigned)((ngroup + kGroupCta - 1) / kGroupCta);           // one lane per group
     k_index_spec<<<grid, 256, 0, st>>>(body, body_len, nseg, w.paths, w.exits);
     k_group_init<<<wgrid, kGroupCta, 0, st>>>(body, body_len, nseg, ngroup, w.paths, w.exits, w.g_entry, w.g_exit, w.g_vis,
-                                        w.claim, w.entry, getenv("SNAPPY_B200_K0_NO_RUNUP") == nullptr,
+                                        w.claim, w.entry,
                                         // mostly incompressible (stream >= 80 % of the output): chains of maximal literals
-                                        !open_end && getenv("SNAPPY_B200_K0_NO_RUNUP") == nullptr &&
-                                            stream_bytes / 4 >= total_out / 5);
+                                        !open_end && stream_bytes / 4 >= total_out / 5);
     *launches += 2;
     const uint64_t max_rounds = ngroup + 2 + kMaxBatch;
     const uint32_t *unresolved = nullptr; // flag of the last round run, when nothing proves convergence
@@ -973,9 +968,8 @@ cudaError_t run_index(const uint8_t *d_stream, uint64_t stream_bytes, uint64_t b
     // small streams do not pay for a full batch of launches
     batch = (uint32_t)std::min<uint64_t>(batch, ngroup + 1);
     // Two claim buffers: round 0 is scatter + k_group_apply (one warp per group: the first round moves most
-    // groups); from round 1 on one fused kernel per round applies the claims of one buffer and scatters those of
-    // the next round into the other.  SNAPPY_B200_K0_UNFUSED=1 keeps the two-kernel rounds (A/B).
-    static const bool unfused = getenv("SNAPPY_B200_K0_UNFUSED") != nullptr;
+    // groups) + scatter of the claims of round 1; from round 1 on one fused kernel per round applies the claims of
+    // one buffer and scatters those of the next round into the other.
     unsigned long long *claim[2] = {w.claim, w.claim + align_up(ngroup + 1, 32)};
     if ((e = cudaMemsetAsync(claim[1], 0xff, (ngroup + 1) * 8, st)) != cudaSuccess) // kNone
         return e;
@@ -986,18 +980,11 @@ cudaError_t run_index(const uint8_t *d_stream, uint64_t stream_bytes, uint64_t b
         for (uint32_t k = 0; k < batch; ++k) {
             const uint32_t *prev = k ? w.changed + k - 1 : nullptr;
             if (round + k == 0) {
-                k_group_scatter<<<ggrid, 128, 0, st>>>(body, body_len, ngroup, w.g_entry, w.g_exit, claim[0], nullptr);
+                k_group_scatter<<<ggrid, 128, 0, st>>>(body, body_len, ngroup, w.g_entry, w.g_exit, claim[0]);
                 k_group_apply<<<wgrid, kGroupCta, 0, st>>>(body, body_len, nseg, ngroup, w.paths, w.exits, w.g_entry,
                                                            w.g_exit, w.g_vis, claim[0], w.changed + k, w.entry);
-                if (!unfused) // the claims of round 1
-                    k_group_scatter<<<ggrid, 128, 0, st>>>(body, body_len, ngroup, w.g_entry, w.g_exit, claim[0], nullptr);
+                k_group_scatter<<<ggrid, 128, 0, st>>>(body, body_len, ngroup, w.g_entry, w.g_exit, claim[0]);
                 *launches += 3;
-            } else if (unfused) {
-                k_group_scatter<<<ggrid, 128, 0, st>>>(body, body_len, ngroup, w.g_entry, w.g_exit, claim[0], prev);
-                k_group_apply32<<<wgrid32, kGroupCta, 0, st>>>(body, body_len, nseg, ngroup, w.paths, w.exits,
-                                                               w.g_entry, w.g_exit, w.g_vis, claim[0], w.changed + k,
-                                                               prev, w.entry, nullptr);
-                *launches += 2;
             } else {
                 k_group_apply32<<<wgrid32, kGroupCta, 0, st>>>(body, body_len, nseg, ngroup, w.paths, w.exits,
                                                                w.g_entry, w.g_exit, w.g_vis, claim[cur], w.changed + k,

@@ -7,7 +7,7 @@ strict_ref alone, never by how the stream was made.
 
 CPU part: the generators, the strict reference and the oracle agree, every family hits what it aims at.
 GPU part: one child process per setting of the switches the library reads once per process
-(SNAPPY_B200_DECODER, SNAPPY_B200_DECODE_PRODUCE, SNAPPY_B200_PIECE_MIB); each decodes every stream through
+(SNAPPY_B200_DECODER, SNAPPY_B200_PIECE_MIB); each decodes every stream through
 every entry point and reports the calls that broke the contract as one JSON line.
 
 Regression cases of the bugs this suite found (named by case id):
@@ -379,11 +379,10 @@ SETTINGS = {
     "auto": {},
     "seg": {"SNAPPY_B200_DECODER": "seg"},
     "tile": {"SNAPPY_B200_DECODER": "tile"},
-    "seg-follow": {"SNAPPY_B200_DECODER": "seg", "SNAPPY_B200_DECODE_PRODUCE": "follow"},
     "pieces-1mib": {"SNAPPY_B200_PIECE_MIB": "1", "SNAPPY_B200_PIECE_START_MIB": "1"},
 }
-_SWITCHES = ("SNAPPY_B200_DECODER", "SNAPPY_B200_DECODE_PRODUCE", "SNAPPY_B200_PIECE_MIB",
-             "SNAPPY_B200_PIECE_START_MIB", "SNAPPY_B200_PIECE_GROWTH", "SNAPPY_B200_DEVICES")
+_SWITCHES = ("SNAPPY_B200_DECODER", "SNAPPY_B200_PIECE_MIB", "SNAPPY_B200_PIECE_START_MIB",
+             "SNAPPY_B200_PIECE_GROWTH", "SNAPPY_B200_DEVICES")
 
 
 def _run_child(code, args, env_over, timeout=900):

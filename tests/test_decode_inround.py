@@ -1,7 +1,6 @@
-"""k_decode_seg's two ways of resolving a copy whose source byte is produced in the same 32-byte round
-(pointer doubling over lanes, and the follow-back loop behind SNAPPY_B200_DECODE_PRODUCE=follow) on
-streams full of short copy chains, against the oracle decoder and the generator's own output.
-Every stream has more than 32 blocks, so the segment decoder runs and not the tile decoder."""
+"""k_decode_seg's pointer doubling over lanes, which resolves a copy whose source byte is produced in the
+same 32-byte round, on streams full of short copy chains, against the oracle decoder and the generator's
+own output.  Every stream has more than 32 blocks, so the segment decoder runs and not the tile decoder."""
 import os
 import subprocess
 import sys
@@ -117,15 +116,10 @@ def chain_streams(tmp_path_factory, oracle):
     return path
 
 
-@pytest.mark.parametrize("produce", ["shuffle", "follow"])
-def test_inround_chains_both_producers(chain_streams, produce):
-    """SNAPPY_B200_DECODE_PRODUCE is read once per process, so each setting decodes in a process of its own."""
+def test_inround_chains(chain_streams):
+    """Decodes in a process of its own, with the decoder picked by input size (SNAPPY_B200_DECODER unset)."""
     env = dict(os.environ)
     env.pop("SNAPPY_B200_DECODER", None)
-    if produce == "follow":
-        env["SNAPPY_B200_DECODE_PRODUCE"] = "follow"
-    else:
-        env.pop("SNAPPY_B200_DECODE_PRODUCE", None)
     r = subprocess.run([sys.executable, "-c", _CHILD % ROOT, str(chain_streams)], capture_output=True, text=True,
                        timeout=600, env=env)
     assert r.returncode == 0 and "OK" in r.stdout, (r.stdout[-2000:], r.stderr[-3000:])

@@ -310,18 +310,6 @@ def test_selftest_driver():
 
 
 @pytest.mark.gpu
-def test_shared_memory_table_variant(oracle, monkeypatch):
-    """The A/B switch SNAPPY_B200_SMEM_TABLES=1 (tables in shared memory, one CTA per block: the
-    kernels the global-memory tables replaced) must give the same bytes."""
-    monkeypatch.setenv("SNAPPY_B200_SMEM_TABLES", "1")
-    specs = _fuzz_specs()[::7] + ["corpus:text:3:0:300000", "corpus:lowent:3:0:300000", "corpus:mixed:3:0:3200000"]
-    for spec in specs:
-        data = datasets.gen(spec)
-        for mode, fn in ((0, api.snappy_compress), (1, api.snappy_compress_bst)):
-            _assert_same(fn(data), oracle.compress(data, mode), f"{spec} mode {mode} (shared-memory tables)")
-
-
-@pytest.mark.gpu
 def test_side_index_host_api(oracle, monkeypatch):
     """SURVEY 8f-4: the optional side index.  The stream is unchanged, the index equals the
     oracle's block index, the indexed decoder (no K0) inverts it, and a wrong index is reported."""

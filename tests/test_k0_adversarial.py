@@ -14,8 +14,8 @@ On these streams it needs about that many, which is what this suite pins down:
     16 384 rounds with ST_UNRESOLVED (reported as a corrupt stream) although the stream is valid.
 
 Sizes put ngroup on the edges of the 16 / 48 / 64 batch schedule of the adaptive mode.  GPU tests run one child
-process per K0 setting (SNAPPY_B200_K0_UNFUSED, SNAPPY_B200_K0_NO_RUNUP, SNAPPY_B200_DECODER), which the
-library reads once per process.
+process per setting of SNAPPY_B200_DECODER (the decoder picked by size, and the tile decoder), which the library
+reads once per process.
 """
 from __future__ import annotations
 
@@ -288,13 +288,10 @@ print("FAILS " + json.dumps(fails))
 
 SETTINGS = {
     "default": ({"K0ADV_CLI": "1"}, max(NGROUPS)),
-    "unfused": ({"SNAPPY_B200_K0_UNFUSED": "1"}, max(NGROUPS)),
-    "no-runup": ({"SNAPPY_B200_K0_NO_RUNUP": "1"}, max(NGROUPS)),
     "tile": ({"SNAPPY_B200_DECODER": "tile"}, SMALL),
 }
-_SWITCHES = ("SNAPPY_B200_DECODER", "SNAPPY_B200_DECODE_PRODUCE", "SNAPPY_B200_PIECE_MIB",
-             "SNAPPY_B200_PIECE_START_MIB", "SNAPPY_B200_PIECE_GROWTH", "SNAPPY_B200_DEVICES",
-             "SNAPPY_B200_K0_UNFUSED", "SNAPPY_B200_K0_NO_RUNUP")
+_SWITCHES = ("SNAPPY_B200_DECODER", "SNAPPY_B200_PIECE_MIB", "SNAPPY_B200_PIECE_START_MIB",
+             "SNAPPY_B200_PIECE_GROWTH", "SNAPPY_B200_DEVICES")
 
 
 def _run_child(code, args, env_over, timeout=1800):
