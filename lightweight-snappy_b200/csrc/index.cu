@@ -5,6 +5,13 @@
 // (src/snappy_compression.c:334-336 just appends blocks).  A sequential tag walk over a
 // gigabyte is hopeless on a GPU, so the walk is made parallel by speculation:
 //
+//   0  k_literal_cand  incompressible blocks are stored as maximal literals, "f4 ff ff" + 65 536 bytes,
+//      k_literal_cover whose payload holds no element.  Before any tag walk, every 8 KiB group records
+//                      the first and last "f4 ff ff" in it (a candidate header), and every group that
+//                      lies inside the payload of an accepted candidate is marked covered: its segments
+//                      are not walked (A), it is not resolved (B) and it starts out dead.  The group
+//                      that holds the end of an accepted literal takes that offset as its first belief.
+//                      The candidates are guesses like every other belief: a wrong one costs rounds.
 //   A  k_index_spec    the stream body is cut into 128-byte segments, one thread each.  Every
 //                      thread walks elements from the first byte of its segment as if an
 //                      element started there, remembers the visited offsets in a 128-bit map
@@ -131,12 +138,129 @@ __device__ __forceinline__ uint64_t walk(const uint8_t *__restrict__ body, uint6
     return e;
 }
 
+// ---- groups of kGroup segments ------------------------------------------------------------
+constexpr uint32_t kGroup = 64;                   // segments per group
+constexpr uint64_t kGroupBytes = kGroup * kSeg;   // 8 KiB of stream
+constexpr uint32_t kGDead = 0x80000000u;          // g_entry bit 31: no element starts in this group
+constexpr uint32_t kGMark = 0xffffffu;            // claim payload: "a literal jumps over you"
+constexpr uint32_t kGUnwalked = 0xfffffeu;        // g_entry of a covered group: no claim carries this offset
+constexpr uint32_t kLitNone = 0xffffffffu;        // g_lit: nothing known from the maximal literals
+constexpr uint32_t kLitCovered = 0xfffffffeu;     // g_lit: inside the payload of an accepted maximal literal
+                                                  //        (else g_lit = offset in the group where one ends)
+
+// ---- maximal literals (0) -------------------------------------------------------------------
+constexpr int kGroupCta = 128;                 // 4 warps = 4 groups per CTA (one warp per group)
+constexpr uint32_t kNoCand = 0xffffffffu;
+
+// g_cand[g] = offsets in group g of the first and last candidate header: a position p where "f4 ff ff"
+// starts and p + 65 539 <= body_len (kNoCand: none).  In the open-ended mode body_len is what has been
+// uploaded, so a literal that is not all there yet is no candidate.  The 8 KiB are read with coalesced
+// word loads; every lane checks the four positions of its word against the word after it, which lies
+// before body_len - 65 536 as well.
+__global__ void __launch_bounds__(kGroupCta) k_literal_cand(const uint8_t *__restrict__ body, uint64_t body_len,
+                                                            uint64_t ngroup, uint2 *__restrict__ g_cand)
+{
+    const uint64_t g = blockIdx.x * (uint64_t)(kGroupCta / 32) + (threadIdx.x >> 5);
+    if (g >= ngroup)
+        return;
+    const uint32_t lane = threadIdx.x & 31;
+    const uint64_t g_lo = g * kGroupBytes;
+    const uint64_t lim = body_len >= kMaxLiteralElemBytes ? body_len - kMaxLiteralElemBytes + 1 : 0; // positions < lim
+    const uint32_t n = g_lo < lim ? (uint32_t)min(kGroupBytes, lim - g_lo) : 0;
+    uint32_t first = kNoCand, last = 0; // (last: offset + 1)
+    if (n) {
+        const uint8_t *src = body + g_lo;
+        const uint32_t a = (uint32_t)reinterpret_cast<uintptr_t>(src) & 3u;
+        const uint32_t *wp = reinterpret_cast<const uint32_t *>(src - a); // (same allocation: it is 4-aligned)
+        const uint32_t nw = (a + n + 3u) >> 2;
+#pragma unroll 4
+        for (uint32_t i = lane; i < nw; i += 32) {
+            const uint32_t w0 = __ldg(wp + i), w1 = __ldg(wp + i + 1);
+            if (!__vcmpeq4(__funnelshift_r(w0, w1, 8u), 0xffffffffu))
+                continue; // no 0xff right after any of the four positions (all of text and nearly all else)
+#pragma unroll
+            for (uint32_t k = 0; k < 4; ++k) {
+                const uint32_t off = 4u * i + k - a; // wraps below 0 for the bytes before src
+                if ((__funnelshift_r(w0, w1, 8u * k) & 0xffffffu) == 0xfffff4u && off < n) {
+                    first = min(first, off);
+                    last = max(last, off + 1);
+                }
+            }
+        }
+    }
+    first = __reduce_min_sync(kFull, first);
+    last = __reduce_max_sync(kFull, last);
+    if (lane == 0)
+        g_cand[g] = make_uint2(first, last ? last - 1 : kNoCand);
+}
+
+// A candidate q is accepted unless another candidate p shadows it: p < q < p + 65 539 (q lies in p's payload).
+// The chained successor of a literal sits exactly at p + 65 539 and is not shadowed.  Without the rule a false
+// "f4 ff ff" inside a payload (about one incompressible block in 256) would spread coverage up to 64 KiB into
+// the next, compressible block.  Only the first and last candidate of a group are known, which is all that can
+// shadow: the first of q's group, and the last of the earlier groups the window reaches.
+__device__ __forceinline__ bool literal_accepted(const uint2 *__restrict__ g_cand, uint64_t q)
+{
+    const uint64_t gq = q / kGroupBytes;
+    if (g_cand[gq].x < q - gq * kGroupBytes)
+        return false;
+    const uint64_t lo = q >= kMaxLiteralElemBytes - 1 ? q - (kMaxLiteralElemBytes - 1) : 0; // shadowing p >= lo
+    for (uint64_t h = gq; h-- > lo / kGroupBytes;) {
+        const uint32_t l = g_cand[h].y;
+        if (l != kNoCand && h * kGroupBytes + l >= lo)
+            return false;
+    }
+    return true;
+}
+
+// g_lit[g] for every group, from the candidates of the nine groups before it (one thread per group):
+// kLitCovered when the group holds no candidate and lies inside [p + 3, p + 65 539) of an accepted p; else the
+// offset of p + 65 539 when that falls inside the group; else kLitNone.  Two accepted candidates lie at least
+// 65 539 apart, so at most one literal covers a group or ends in it.
+__global__ void __launch_bounds__(256) k_literal_cover(uint64_t body_len, uint64_t ngroup,
+                                                       const uint2 *__restrict__ g_cand, uint32_t *__restrict__ g_lit)
+{
+    const uint64_t g = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (g >= ngroup)
+        return;
+    const uint64_t g_lo = g * kGroupBytes, g_hi = min(g_lo + kGroupBytes, body_len);
+    const bool has_cand = g_cand[g].x != kNoCand;
+    uint32_t lit = kLitNone;
+    const uint64_t h_lo = g > kMaxLiteralElemBytes / kGroupBytes ? g - 1 - kMaxLiteralElemBytes / kGroupBytes : 0;
+    for (uint64_t h = g; h-- > h_lo;) {
+        const uint2 c = g_cand[h];
+        for (int j = 0; j < 2; ++j) {
+            const uint32_t off = j ? c.y : c.x;
+            if (off == kNoCand)
+                continue;
+            const uint64_t p = h * kGroupBytes + off, end = p + kMaxLiteralElemBytes;
+            if (!has_cand && p + 3 <= g_lo && end >= g_hi && literal_accepted(g_cand, p))
+                lit = kLitCovered;
+            else if (end >= g_lo && end < g_hi && literal_accepted(g_cand, p))
+                lit = (uint32_t)(end - g_lo);
+        }
+    }
+    g_lit[g] = lit;
+}
+
+// exits[t] of a segment that k_index_spec did not walk (a covered group).  Its path is empty and its exit
+// means nothing, and nothing may read them as a walk's result: group_stage walks such a segment before
+// group_resolve sees it, and the group's g_vis is 0 and its g_entry is kGDead | kGUnwalked until then, so
+// every new entry the group is given sends it through group_resolve (and so through group_stage).
+constexpr uint64_t kUnwalked = kNone;
+
 __global__ void __launch_bounds__(256) k_index_spec(const uint8_t *__restrict__ body, uint64_t body_len, uint64_t nseg,
-                                                    uint4 *__restrict__ paths, uint64_t *__restrict__ exits)
+                                                    const uint32_t *__restrict__ g_lit, uint4 *__restrict__ paths,
+                                                    uint64_t *__restrict__ exits)
 {
     const uint64_t t = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     if (t >= nseg)
         return;
+    if (g_lit[t / kGroup] == kLitCovered) {
+        paths[t] = make_uint4(0, 0, 0, 0);
+        exits[t] = kUnwalked;
+        return;
+    }
     const uint64_t lo = t * kSeg;
     const uint64_t hi = min(lo + kSeg, body_len);
     Path p;
@@ -147,16 +271,9 @@ __global__ void __launch_bounds__(256) k_index_spec(const uint8_t *__restrict__ 
     exits[t] = x;
 }
 
-// ---- groups of kGroup segments ------------------------------------------------------------
-constexpr uint32_t kGroup = 64;                   // segments per group
-constexpr uint64_t kGroupBytes = kGroup * kSeg;   // 8 KiB of stream
-constexpr uint32_t kGDead = 0x80000000u;          // g_entry bit 31: no element starts in this group
-constexpr uint32_t kGMark = 0xffffffu;            // claim payload: "a literal jumps over you"
-
 // One warp works on one group.  The group's per-segment records (path map + exit) are staged
 // in shared memory with coalesced loads; the chase itself is a short dependent chain that all
 // lanes execute redundantly on the staged copy.
-constexpr int kGroupCta = 128;                 // 4 warps = 4 groups per CTA
 struct GroupStage {
     uint4 paths[kGroup];
     uint64_t exits[kGroup];
@@ -164,8 +281,11 @@ struct GroupStage {
     uint8_t entry[kGroup];
 };
 
-// Stages the per-segment records of group g.
-__device__ __forceinline__ void group_stage(GroupStage &sm, uint64_t g, uint64_t nseg, const uint4 *__restrict__ paths,
+// Stages the per-segment records of group g.  A segment k_index_spec did not walk (a covered group that
+// has just been given an entry) is walked here from its first byte, as k_index_spec would have done, so
+// that group_resolve only ever sees the records of walks; group_unstage then stores them.
+__device__ __forceinline__ void group_stage(const uint8_t *__restrict__ body, uint64_t body_len, GroupStage &sm,
+                                            uint64_t g, uint64_t nseg, const uint4 *__restrict__ paths,
                                             const uint64_t *__restrict__ exits)
 {
     const uint32_t lane = threadIdx.x & 31;
@@ -173,8 +293,18 @@ __device__ __forceinline__ void group_stage(GroupStage &sm, uint64_t g, uint64_t
 #pragma unroll
     for (uint32_t k = lane; k < kGroup; k += 32) {
         const bool ok = s0 + k < nseg;
-        sm.paths[k] = ok ? paths[s0 + k] : make_uint4(0, 0, 0, 0);
-        sm.exits[k] = ok ? exits[s0 + k] : 0;
+        uint4 pv = ok ? paths[s0 + k] : make_uint4(0, 0, 0, 0);
+        uint64_t x = ok ? exits[s0 + k] : 0;
+        if (x == kUnwalked) {
+            const uint64_t lo = (s0 + k) * kSeg;
+            Path p;
+            p.clear();
+            bool merged;
+            x = walk(body, body_len, lo, min(lo + kSeg, body_len), lo, nullptr, p, merged);
+            pv = make_uint4(p.bits[0], p.bits[1], p.bits[2], p.bits[3]);
+        }
+        sm.paths[k] = pv;
+        sm.exits[k] = x;
     }
     __syncwarp();
 }
@@ -306,62 +436,45 @@ __device__ __forceinline__ uint64_t group_resolve(const uint8_t *__restrict__ bo
     return sm.exits[last];
 }
 
-// Initial state: every group believes an element starts at its first byte.
+// Initial state of every group.  A covered group (inside a maximal literal's payload) starts out dead,
+// unresolved and silent: g_exit = kNone lands in no group, so it publishes no claim until a claim gives it
+// an entry.  Every other group is resolved from its first belief.
 __global__ void __launch_bounds__(kGroupCta) k_group_init(const uint8_t *__restrict__ body, uint64_t body_len,
                                                           uint64_t nseg, uint64_t ngroup, uint4 *__restrict__ paths,
-                                                          uint64_t *__restrict__ exits,
+                                                          uint64_t *__restrict__ exits, const uint32_t *__restrict__ g_lit,
                                                           uint32_t *__restrict__ g_entry, uint64_t *__restrict__ g_exit,
                                                           uint64_t *__restrict__ g_vis,
                                                           unsigned long long *__restrict__ g_claim,
-                                                          uint8_t *__restrict__ entries, int literal_scan)
+                                                          uint8_t *__restrict__ entries)
 {
     __shared__ GroupStage stage[kGroupCta / 32];
     const uint64_t g = blockIdx.x * (uint64_t)(kGroupCta / 32) + (threadIdx.x >> 5);
     if (g >= ngroup)
         return;
-    GroupStage &sm = stage[threadIdx.x >> 5];
-    group_stage(sm, g, nseg, paths, exits);
-    // First belief about where the chain enters this group.  "At its first byte" is right one time in four
-    // on text; the speculative walks of the segments just before the group are a free run-up: follow their
-    // exits (exit of segment s, landing on the recorded path of the segment it falls in, that segment's exit,
-    // ...) from up to three segments back into the group.  Every hop that lands on a recorded path halves the
-    // chance that the walk is still off the true chain.  Only table look-ups, no tag walk; any value read here
-    // is a guess that the relaxation corrects (a neighbour may be rewriting its records meanwhile).
-    uint64_t e0 = g * kGroupBytes;
-    // Incompressible blocks are maximal literals, "f4 ff ff" + 65 536 bytes, and the payload in between
-    // tells nothing: a group that lies right after such a literal looks 65 539 bytes back for the header that
-    // would end inside it.  A hit is strong evidence (24 bits) for an element start, and it turns the chain of
-    // literals of a run of incompressible blocks, which the relaxation can only follow 24 per round, into
-    // local knowledge of every group (random data: 32 -> 10 rounds, K0 4.9 -> 3.1 ms).  The 8 KiB are read
-    // with coalesced word loads, every lane checks the four byte positions of its word against the word after
-    // it.  Reading the stream once more costs 0.15 ms per GiB of mixed data, where it finds nothing: the scan is
-    // only switched on for streams that are mostly incompressible (run_index).
-    uint64_t lit_end = kNone;
-    if (literal_scan && g * kGroupBytes >= kMaxLiteralElemBytes) {
-        const uint64_t g_lo = g * kGroupBytes, g_hi = min(g_lo + kGroupBytes, body_len);
-        const uint32_t lane = threadIdx.x & 31;
-        const uint32_t n = (uint32_t)(g_hi - g_lo); // header positions src .. src + n
-        const uint8_t *src = body + (g_lo - kMaxLiteralElemBytes);
-        const uint32_t a = (uint32_t)reinterpret_cast<uintptr_t>(src) & 3u;
-        const uint32_t *wp = reinterpret_cast<const uint32_t *>(src - a);
-        const uint32_t nw = (a + n + 3u) >> 2; // words that hold a candidate position (<= 2049)
-        uint32_t first = 0xffffffffu;         // position (relative to src) of the first header found by this lane
-#pragma unroll 4
-        for (uint32_t i = lane; i < nw; i += 32) {
-            const uint32_t w0 = __ldg(wp + i), w1 = __ldg(wp + i + 1); // (w1: at most 4 bytes past the last position, still before g_lo)
-#pragma unroll
-            for (uint32_t k = 0; k < 4; ++k) {
-                const uint32_t off = 4u * i + k - a; // wraps below 0 for the bytes before src
-                if ((__funnelshift_r(w0, w1, 8u * k) & 0xffffffu) == 0xfffff4u && off < n)
-                    first = min(first, off);
-            }
+    const uint32_t lit = g_lit[g];
+    if (lit == kLitCovered) {
+        if ((threadIdx.x & 31) == 0) {
+            g_exit[g] = kNone;
+            g_vis[g] = 0;
+            g_entry[g] = kGDead | kGUnwalked;
+            g_claim[g] = kNone;
         }
-        const uint32_t best = __reduce_min_sync(kFull, first);
-        if (best != 0xffffffffu)
-            lit_end = g_lo + best;
+        return;
     }
-    if (lit_end != kNone) {
-        e0 = lit_end;
+    GroupStage &sm = stage[threadIdx.x >> 5];
+    group_stage(body, body_len, sm, g, nseg, paths, exits);
+    // First belief about where the chain enters this group.  Where a maximal literal ends inside the group,
+    // that offset (k_literal_cover: 24 bits of evidence, and the chain of a run of incompressible blocks becomes
+    // local knowledge of every group).  Otherwise "at its first byte" is right one time in four on text; the
+    // speculative walks of the segments just before the group are a free run-up: follow their exits (exit of
+    // segment s, landing on the recorded path of the segment it falls in, that segment's exit, ...) from up to
+    // three segments back into the group.  Every hop that lands on a recorded path halves the chance that the
+    // walk is still off the true chain.  Only table look-ups, no tag walk; any value read here is a guess that
+    // the relaxation corrects (a neighbour may be rewriting its records meanwhile; an unwalked segment's exit,
+    // kUnwalked, lies past the group and is not taken).
+    uint64_t e0 = g * kGroupBytes;
+    if (lit != kLitNone) {
+        e0 += lit;
     } else if (g > 0) {
         const uint64_t g_lo = g * kGroupBytes, g_hi = min(g_lo + kGroupBytes, body_len);
         const uint64_t s_last = g * kGroup - 1;
@@ -511,10 +624,11 @@ __global__ void __launch_bounds__(kGroupCta) k_group_apply(const uint8_t *__rest
     const uint4 pv = paths[sg];
     Path p;
     p.bits[0] = pv.x, p.bits[1] = pv.y, p.bits[2] = pv.z, p.bits[3] = pv.w;
+    // (a covered group that was never resolved has g_vis == 0: it always goes on to group_resolve)
     if (((g_vis[g] >> (sg - g * kGroup)) & 1ull) && p.test((uint32_t)(e - sg * kSeg)))
         return; // same exit, and everything the old chain recorded still holds from here on
     GroupStage &sm = stage[threadIdx.x >> 5];
-    group_stage(sm, g, nseg, paths, exits);
+    group_stage(body, body_len, sm, g, nseg, paths, exits);
     uint64_t vis;
     const uint64_t x = group_resolve(body, body_len, nseg, sm, g, e, vis);
     group_unstage(sm, g, nseg, paths, exits, entries);
@@ -571,6 +685,7 @@ __global__ void __launch_bounds__(kGroupCta) k_group_apply32(const uint8_t *__re
                 const uint4 pv = paths[sg];
                 Path p;
                 p.bits[0] = pv.x, p.bits[1] = pv.y, p.bits[2] = pv.z, p.bits[3] = pv.w;
+                // (g_vis == 0 for a covered group that was never resolved: always heavy)
                 heavy = !(((g_vis[g] >> (sg - g * kGroup)) & 1ull) && p.test((uint32_t)(e - sg * kSeg)));
             }
         }
@@ -584,7 +699,7 @@ __global__ void __launch_bounds__(kGroupCta) k_group_apply32(const uint8_t *__re
         H &= H - 1;
         const uint64_t gg = (uint64_t)src * n_warps + w;
         const uint64_t ee = __shfl_sync(kFull, e, src);
-        group_stage(sm, gg, nseg, paths, exits);
+        group_stage(body, body_len, sm, gg, nseg, paths, exits);
         uint64_t vis;
         const uint64_t x = group_resolve(body, body_len, nseg, sm, gg, ee, vis);
         group_unstage(sm, gg, nseg, paths, exits, entries);
@@ -867,6 +982,8 @@ struct IndexWorkspace {
     uint32_t *g_entry;
     uint64_t *g_exit;
     uint64_t *g_vis;
+    uint2 *g_cand;
+    uint32_t *g_lit;
 };
 
 static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -878,7 +995,7 @@ size_t index_workspace_bytes(uint64_t stream_bytes)
     const uint64_t ngroup = (nseg + kGroup - 1) / kGroup + 1;
     return align_up(nseg * 16, 256) + 3 * align_up(nseg * 8, 256) + align_up(std::max<uint64_t>(nseg, 128) * 8, 256) +
            align_up(ntile * 8, 256) + 256 + 256 +
-           align_up(nseg, 256) + align_up(ngroup * 4, 256) + 2 * align_up(ngroup * 8, 256) + 256;
+           align_up(nseg, 256) + 2 * align_up(ngroup * 4, 256) + 3 * align_up(ngroup * 8, 256) + 256;
 }
 
 static IndexWorkspace carve(void *ws, uint64_t stream_bytes)
@@ -899,7 +1016,9 @@ static IndexWorkspace carve(void *ws, uint64_t stream_bytes)
     const uint64_t ngroup = (nseg + kGroup - 1) / kGroup + 1;
     w.g_entry = reinterpret_cast<uint32_t *>(p), p += align_up(ngroup * 4, 256);
     w.g_exit = reinterpret_cast<uint64_t *>(p), p += align_up(ngroup * 8, 256);
-    w.g_vis = reinterpret_cast<uint64_t *>(p);
+    w.g_vis = reinterpret_cast<uint64_t *>(p), p += align_up(ngroup * 8, 256);
+    w.g_cand = reinterpret_cast<uint2 *>(p), p += align_up(ngroup * 8, 256);
+    w.g_lit = reinterpret_cast<uint32_t *>(p);
     return w;
 }
 
@@ -955,12 +1074,12 @@ cudaError_t run_index(const uint8_t *d_stream, uint64_t stream_bytes, uint64_t b
     const unsigned ggrid = (unsigned)((ngroup + 127) / 128);                       // one thread per group
     const unsigned wgrid = (unsigned)((ngroup + kGroupCta / 32 - 1) / (kGroupCta / 32)); // one warp per group
     const unsigned wgrid32 = (unsigned)((ngroup + kGroupCta - 1) / kGroupCta);           // one lane per group
-    k_index_spec<<<grid, 256, 0, st>>>(body, body_len, nseg, w.paths, w.exits);
-    k_group_init<<<wgrid, kGroupCta, 0, st>>>(body, body_len, nseg, ngroup, w.paths, w.exits, w.g_entry, w.g_exit, w.g_vis,
-                                        w.claim, w.entry,
-                                        // mostly incompressible (stream >= 80 % of the output): chains of maximal literals
-                                        !open_end && stream_bytes / 4 >= total_out / 5);
-    *launches += 2;
+    k_literal_cand<<<wgrid, kGroupCta, 0, st>>>(body, body_len, ngroup, w.g_cand);
+    k_literal_cover<<<(unsigned)((ngroup + 255) / 256), 256, 0, st>>>(body_len, ngroup, w.g_cand, w.g_lit);
+    k_index_spec<<<grid, 256, 0, st>>>(body, body_len, nseg, w.g_lit, w.paths, w.exits);
+    k_group_init<<<wgrid, kGroupCta, 0, st>>>(body, body_len, nseg, ngroup, w.paths, w.exits, w.g_lit, w.g_entry,
+                                              w.g_exit, w.g_vis, w.claim, w.entry);
+    *launches += 4;
     const uint64_t max_rounds = ngroup + 2 + kMaxBatch;
     const uint32_t *unresolved = nullptr; // flag of the last round run, when nothing proves convergence
     uint32_t batch = fixed_rounds ? std::min<uint32_t>(fixed_rounds, kMaxBatch) : 16;
