@@ -46,6 +46,13 @@ extern "C" {
 
 #define SNAPPY_B200_MODE_HASH 0 /* src/snappy_compression.c */
 #define SNAPPY_B200_MODE_BST 1  /* src/snappy_compression_tree.c */
+/* A parse designed for the GPU: candidates for every position of a block are found in parallel and short
+ * slices of the block are parsed independently (csrc/parallel_parse.h defines it).  The stream is valid Snappy
+ * in the reference's format (varint, then 64 KiB blocks; no element leaves its block, so every decoder here
+ * takes it on its fast path), the same input always gives the same bytes (whatever the stream, the device or
+ * the device count), but it is NOT byte-identical to the reference's: use MODE_HASH or MODE_BST for that.
+ * Its compression workspace is larger (snappy_b200_compress_workspace_bytes(n, mode) accounts for it). */
+#define SNAPPY_B200_MODE_PARALLEL 2
 
 #define SNAPPY_B200_OK 0
 #define SNAPPY_B200_ERR_CUDA (-1)     /* CUDA runtime / driver error, or no device */
@@ -196,6 +203,8 @@ int snappy_b200_decompress_host_indexed_multi(const void *stream, uint64_t strea
  * own file next to the unchanged stream -- "SNPIDX1\0", u64 uncompressed bytes, u64 n_blocks,
  * then n_blocks + 1 u64 stream offsets, all little-endian.  Same FILE* ownership rules as the
  * drop-in calls (caller opens and closes).                                                */
+/* index_out may be NULL: then this is the plain FILE* compressor, for every mode (the reference's snappy_compress
+ * and snappy_compress_bst are MODE_HASH and MODE_BST only).                                                    */
 int snappy_b200_compress_file_indexed(FILE *in, unsigned long long input_size, int mode, FILE *out, FILE *index_out);
 int snappy_b200_decompress_file_indexed(FILE *in, FILE *index_in, FILE *out);
 /* FILE* -> FILE* decompression with the stream and the output device-resident and only a ring of three

@@ -11,6 +11,9 @@ src/snappy_compression_tree.h:10, src/snappy_decompression.h:15):
     snappy_compress(data)      -> stream   (hash-table path)
     snappy_compress_bst(data)  -> stream   (BST / exact-key path)
     snappy_decompress(stream)  -> data
+
+MODE_PARALLEL selects the block-parallel parse: a valid Snappy stream in the same format that
+every decoder reads, deterministic, but not byte-identical to the reference's.
 """
 from __future__ import annotations
 
@@ -26,7 +29,7 @@ CLI_PATH = os.path.join(HERE, "snappy_b200")
 
 BLOCK = 65536
 SLOT_STRIDE = 66560
-MODE_HASH, MODE_BST = 0, 1
+MODE_HASH, MODE_BST, MODE_PARALLEL = 0, 1, 2
 OK = 0
 ERR_CUDA, ERR_ARG, ERR_CAPACITY, ERR_CORRUPT, ERR_FRAMING, ERR_IO, ERR_CHECKSUM = -1, -2, -3, -4, -5, -6, -7
 ST_CAPACITY, ST_CORRUPT, ST_FRAMING, ST_CHECKSUM = 1, 2, 4, 16
@@ -276,7 +279,8 @@ class DeviceCodec:
     """Pre-allocated device buffers for repeated device-resident calls on one size class.
 
     All tensors live on the current CUDA device; calls are enqueued on torch's current
-    stream and are asynchronous.  `status` / `out_bytes` are device scalars: read them
+    stream and are asynchronous.  The workspace fits every mode, MODE_PARALLEL included, whose
+    candidate offsets take 2 bytes per byte of max_bytes on top of what the other modes need.  `status` / `out_bytes` are device scalars: read them
     (which synchronises) when the result is needed.
     """
 
@@ -289,11 +293,11 @@ class DeviceCodec:
         nb = block_count(max_bytes)
         L = lib()
         self.comp_capacity = max(int(L.snappy_b200_max_compressed_bytes(max_bytes)), 16)
-        ws = max(int(L.snappy_b200_compress_workspace_bytes(max_bytes, MODE_BST)),
+        ws = max(*(int(L.snappy_b200_compress_workspace_bytes(max_bytes, m)) for m in (MODE_BST, MODE_PARALLEL)),
                  int(L.snappy_b200_index_workspace_bytes(self.comp_capacity)),
                  int(L.snappy_b200_decompress_workspace_bytes(self.comp_capacity, max_bytes)),
                  int(L.snappy_b200_decompress_async_workspace_bytes(self.comp_capacity, max_bytes)),
-                 int(L.snappy_b200_frame_compress_workspace_bytes(max_bytes, MODE_BST)))
+                 *(int(L.snappy_b200_frame_compress_workspace_bytes(max_bytes, m)) for m in (MODE_BST, MODE_PARALLEL)))
         self.workspace = torch.empty(ws + 256, dtype=torch.uint8, device=self.device)
         self.stream_buf = torch.empty(self.comp_capacity + 256, dtype=torch.uint8, device=self.device)
         self.block_offsets = torch.zeros(nb + 1, dtype=torch.int64, device=self.device)

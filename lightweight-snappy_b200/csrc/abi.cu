@@ -9,9 +9,10 @@
 #include "common.cuh"
 
 namespace sb200 {
-cudaError_t launch_compress(const uint8_t *, uint64_t, int, uint8_t *, uint32_t *, uint2 *, uint32_t *, cudaStream_t,
-                            uint64_t *);
+cudaError_t launch_compress(const uint8_t *, uint64_t, int, uint8_t *, uint32_t *, uint2 *, uint32_t *, uint16_t *,
+                            cudaStream_t, uint64_t *);
 size_t compress_records_bytes(uint64_t);
+size_t parallel_cand_bytes(uint64_t);
 cudaError_t launch_compact(const uint8_t *, const uint32_t *, uint64_t, uint64_t, uint64_t, int, uint8_t *, uint64_t,
                            uint64_t *, uint64_t *, uint32_t *, cudaStream_t, uint64_t *);
 cudaError_t launch_decode(const uint8_t *, const uint64_t *, uint64_t, uint64_t, uint8_t *, uint32_t *, cudaStream_t,
@@ -54,16 +55,18 @@ struct CompressWorkspace {
     uint32_t *sizes;    // compressed size of every block
     uint32_t *nrec;     // records of every block
     uint64_t *offsets;  // stream offset of every block (when the caller does not want them)
+    uint16_t *cand;     // SNAPPY_B200_MODE_PARALLEL only: the candidate offset of every input byte
 };
 
-static size_t compress_ws_bytes(uint64_t n_bytes)
+static size_t compress_ws_bytes(uint64_t n_bytes, int mode)
 {
     const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
-    return align_up(nb * (size_t)kSlot + 64, 256) + align_up(compress_records_bytes(nb) + 64, 256) +
-           2 * align_up(nb * 4 + 4, 256) + align_up((nb + 1) * 8, 256);
+    const size_t base = align_up(nb * (size_t)kSlot + 64, 256) + align_up(compress_records_bytes(nb) + 64, 256) +
+                        2 * align_up(nb * 4 + 4, 256) + align_up((nb + 1) * 8, 256);
+    return mode == SNAPPY_B200_MODE_PARALLEL ? base + align_up(parallel_cand_bytes(nb), 256) : base;
 }
 
-static CompressWorkspace carve_compress(void *ws, uint64_t n_bytes)
+static CompressWorkspace carve_compress(void *ws, uint64_t n_bytes, int mode)
 {
     const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
     uint8_t *p = static_cast<uint8_t *>(ws);
@@ -72,21 +75,22 @@ static CompressWorkspace carve_compress(void *ws, uint64_t n_bytes)
     w.recs = reinterpret_cast<uint2 *>(p), p += align_up(compress_records_bytes(nb) + 64, 256);
     w.sizes = reinterpret_cast<uint32_t *>(p), p += align_up(nb * 4 + 4, 256);
     w.nrec = reinterpret_cast<uint32_t *>(p), p += align_up(nb * 4 + 4, 256);
-    w.offsets = reinterpret_cast<uint64_t *>(p);
+    w.offsets = reinterpret_cast<uint64_t *>(p), p += align_up((nb + 1) * 8, 256);
+    w.cand = mode == SNAPPY_B200_MODE_PARALLEL ? reinterpret_cast<uint16_t *>(p) : nullptr;
     return w;
 }
 
 // The framed compressor's workspace: the raw compressor's, then the masked CRC and the chunk size of every block.
-static size_t frame_ws_bytes(uint64_t n_bytes)
+static size_t frame_ws_bytes(uint64_t n_bytes, int mode)
 {
     const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
-    return compress_ws_bytes(n_bytes) + 2 * align_up(nb * 4 + 4, 256);
+    return compress_ws_bytes(n_bytes, mode) + 2 * align_up(nb * 4 + 4, 256);
 }
 
-static void carve_frame(void *ws, uint64_t n_bytes, uint32_t **crcs, uint32_t **fsizes)
+static void carve_frame(void *ws, uint64_t n_bytes, int mode, uint32_t **crcs, uint32_t **fsizes)
 {
     const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
-    uint8_t *p = static_cast<uint8_t *>(ws) + compress_ws_bytes(n_bytes);
+    uint8_t *p = static_cast<uint8_t *>(ws) + compress_ws_bytes(n_bytes, mode);
     *crcs = reinterpret_cast<uint32_t *>(p);
     *fsizes = reinterpret_cast<uint32_t *>(p + align_up(nb * 4 + 4, 256));
 }
@@ -116,12 +120,19 @@ static int status_to_error(uint32_t st)
 }
 
 int fail_msg(int code, const char *msg) { return fail(code, "%s", msg); }
+// The one place that decides which compression modes exist: SNAPPY_B200_OK, or SNAPPY_B200_ERR_ARG with the message set.
+int check_mode(int mode)
+{
+    if (mode == SNAPPY_B200_MODE_HASH || mode == SNAPPY_B200_MODE_BST || mode == SNAPPY_B200_MODE_PARALLEL)
+        return SNAPPY_B200_OK;
+    return fail(SNAPPY_B200_ERR_ARG, "unknown mode %d", mode);
+}
 void clear_error() { g_err[0] = 0; } // every public entry point starts clean: a stale message is never reported twice
 int cuda_fail_msg(cudaError_t e, const char *what) { return cuda_fail(e, what); }
 int status_error(uint32_t st) { return status_to_error(st); }
-size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed)
+size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed, int mode)
 {
-    return framed ? frame_ws_bytes(n_bytes) : compress_ws_bytes(n_bytes);
+    return framed ? frame_ws_bytes(n_bytes, mode) : compress_ws_bytes(n_bytes, mode);
 }
 void add_launches(uint64_t n) { g_launches += n; }
 
@@ -162,12 +173,13 @@ cudaError_t compress_chunk(const uint8_t *d_in, uint64_t chunk_bytes, uint64_t v
                            uint32_t *d_status, void *d_workspace, cudaStream_t st)
 {
     const uint64_t nb = (chunk_bytes + kBlock - 1) / kBlock;
-    CompressWorkspace w = carve_compress(d_workspace, chunk_bytes);
+    CompressWorkspace w = carve_compress(d_workspace, chunk_bytes, mode);
     uint64_t launches = 0;
-    cudaError_t e = launch_compress(d_in, chunk_bytes, mode, w.scratch, w.sizes, w.recs, w.nrec, st, &launches);
+    cudaError_t e =
+        launch_compress(d_in, chunk_bytes, mode, w.scratch, w.sizes, w.recs, w.nrec, w.cand, st, &launches);
     if (e == cudaSuccess && framed) {
         uint32_t *crcs, *fsizes;
-        carve_frame(d_workspace, chunk_bytes, &crcs, &fsizes);
+        carve_frame(d_workspace, chunk_bytes, mode, &crcs, &fsizes);
         e = launch_frame_compact(d_in, chunk_bytes, w.scratch, w.sizes, crcs, fsizes, identifier ? 1 : 0, d_out,
                                  out_capacity, w.offsets, d_out_bytes, d_status, st, &launches);
     } else if (e == cudaSuccess) {
@@ -181,7 +193,7 @@ cudaError_t compress_chunk(const uint8_t *d_in, uint64_t chunk_bytes, uint64_t v
 // The block offsets (relative to the chunk's output) compress_chunk left in its workspace: nb + 1 entries.
 const uint64_t *compress_chunk_offsets(void *d_workspace, uint64_t chunk_bytes)
 {
-    return carve_compress(d_workspace, chunk_bytes).offsets;
+    return carve_compress(d_workspace, chunk_bytes, SNAPPY_B200_MODE_HASH).offsets; // (the same for every mode)
 }
 
 } // namespace sb200
@@ -214,8 +226,7 @@ uint64_t snappy_b200_max_compressed_bytes(uint64_t n_bytes)
 
 size_t snappy_b200_compress_workspace_bytes(uint64_t n_bytes, int mode)
 {
-    (void)mode;
-    return compress_ws_bytes(n_bytes);
+    return compress_ws_bytes(n_bytes, mode);
 }
 
 int snappy_b200_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode, uint8_t *d_out, uint64_t out_capacity,
@@ -223,14 +234,15 @@ int snappy_b200_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode,
                                 void *d_workspace, size_t workspace_bytes, void *stream)
 {
     clear_error();
-    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
-        return fail(SNAPPY_B200_ERR_ARG, "unknown mode %d", mode);
+    if (check_mode(mode) != SNAPPY_B200_OK)
+        return SNAPPY_B200_ERR_ARG;
     if (!d_out_bytes || !d_status || (n_bytes && (!d_in || !d_out || !d_workspace)))
         return fail(SNAPPY_B200_ERR_ARG, "null pointer argument");
     if (!aligned16(d_in) || !aligned16(d_out) || !aligned16(d_workspace))
         return fail(SNAPPY_B200_ERR_ARG, "d_in, d_out and d_workspace must be 16-byte aligned");
-    if (workspace_bytes < compress_ws_bytes(n_bytes))
-        return fail(SNAPPY_B200_ERR_ARG, "workspace too small: %zu < %zu", workspace_bytes, compress_ws_bytes(n_bytes));
+    if (workspace_bytes < compress_ws_bytes(n_bytes, mode))
+        return fail(SNAPPY_B200_ERR_ARG, "workspace too small: %zu < %zu", workspace_bytes,
+                    compress_ws_bytes(n_bytes, mode));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
     cudaError_t e = cudaMemsetAsync(d_status, 0, sizeof(uint32_t), st);
@@ -242,9 +254,9 @@ int snappy_b200_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode,
             e = cudaMemsetAsync(d_block_offsets, 0, sizeof(uint64_t), st);
         return e == cudaSuccess ? SNAPPY_B200_OK : cuda_fail(e, "cudaMemsetAsync");
     }
-    CompressWorkspace w = carve_compress(d_workspace, n_bytes);
+    CompressWorkspace w = carve_compress(d_workspace, n_bytes, mode);
     uint64_t launches = 0;
-    e = launch_compress(d_in, n_bytes, mode, w.scratch, w.sizes, w.recs, w.nrec, st, &launches);
+    e = launch_compress(d_in, n_bytes, mode, w.scratch, w.sizes, w.recs, w.nrec, w.cand, st, &launches);
     if (e == cudaSuccess)
         e = launch_compact(w.scratch, w.sizes, nb, n_bytes, host_varint_len(n_bytes), 1, d_out, out_capacity,
                            d_block_offsets ? d_block_offsets : w.offsets, d_out_bytes, d_status, st, &launches);
@@ -261,8 +273,7 @@ uint64_t snappy_b200_frame_max_compressed_bytes(uint64_t n_bytes)
 
 size_t snappy_b200_frame_compress_workspace_bytes(uint64_t n_bytes, int mode)
 {
-    (void)mode;
-    return frame_ws_bytes(n_bytes);
+    return frame_ws_bytes(n_bytes, mode);
 }
 
 int snappy_b200_frame_compress_device(const uint8_t *d_in, uint64_t n_bytes, int mode, uint8_t *d_out,
@@ -270,14 +281,14 @@ int snappy_b200_frame_compress_device(const uint8_t *d_in, uint64_t n_bytes, int
                                       void *d_workspace, size_t workspace_bytes, void *stream)
 {
     clear_error();
-    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
-        return fail(SNAPPY_B200_ERR_ARG, "unknown mode %d", mode);
+    if (check_mode(mode) != SNAPPY_B200_OK)
+        return SNAPPY_B200_ERR_ARG;
     if (!d_out_bytes || !d_status || !d_out || !d_workspace || (n_bytes && !d_in))
         return fail(SNAPPY_B200_ERR_ARG, "null pointer argument");
     if (!aligned16(d_in) || !aligned16(d_out) || !aligned16(d_workspace))
         return fail(SNAPPY_B200_ERR_ARG, "d_in, d_out and d_workspace must be 16-byte aligned");
-    if (workspace_bytes < frame_ws_bytes(n_bytes))
-        return fail(SNAPPY_B200_ERR_ARG, "workspace too small: %zu < %zu", workspace_bytes, frame_ws_bytes(n_bytes));
+    if (workspace_bytes < frame_ws_bytes(n_bytes, mode))
+        return fail(SNAPPY_B200_ERR_ARG, "workspace too small: %zu < %zu", workspace_bytes, frame_ws_bytes(n_bytes, mode));
     if ((n_bytes + kBlock - 1) / kBlock > 0x7fffffffull)
         return fail(SNAPPY_B200_ERR_ARG, "input too large");
     cudaStream_t st = static_cast<cudaStream_t>(stream);

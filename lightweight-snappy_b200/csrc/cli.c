@@ -1,5 +1,6 @@
-/* cli.c -- `snappy [-c|-b|-d] [-r] infile outfile`, the reference's command line
- * (src/cmd.c:19-28, :56-105) in front of libsnappy_b200.so.  Same options and defaults;
+/* cli.c -- `snappy [-c|-b|-p|-d] [-r] infile outfile`, the reference's command line
+ * (src/cmd.c:19-28, :56-105) in front of libsnappy_b200.so.  Same options and defaults, and -p for
+ * SNAPPY_B200_MODE_PARALLEL;
  * -r reports wall-clock time and throughput on the UNCOMPRESSED size for both directions
  * (the reference used CPU time and the compressed size, SURVEY.md Q9).                   */
 #define _POSIX_C_SOURCE 200809L
@@ -18,9 +19,10 @@
 
 static void usage(void)
 {
-    fprintf(stderr, "snappy [-c|-d|-b] [-r] [-i|-f] [infile] [outfile]\n"
+    fprintf(stderr, "snappy [-c|-d|-b|-p] [-r] [-i|-f] [infile] [outfile]\n"
                     "-c compress (hash table)\n"
                     "-b compress (exact-key / BST match finder)\n"
+                    "-p compress (block-parallel parse: valid Snappy, not byte-identical to -c)\n"
                     "-d decompress\n"
                     "-r print sizes, ratio, time and throughput\n"
                     "-i side index: compress also writes <outfile>.idx (block offsets; the stream is\n"
@@ -47,14 +49,15 @@ static double now(void)
 
 int main(int argc, char *argv[])
 {
-    enum { COMPRESS, COMPRESS_BST, UNCOMPRESS } mode = COMPRESS;
+    enum { COMPRESS, COMPRESS_BST, COMPRESS_PARALLEL, UNCOMPRESS } mode = COMPRESS;
     int report = 0, use_index = 0, framed = 0, opt;
     if (argc < 4)
         usage();
-    while ((opt = getopt(argc, argv, "cbdrif")) != -1) {
+    while ((opt = getopt(argc, argv, "cbpdrif")) != -1) {
         switch (opt) {
         case 'c': mode = COMPRESS; break;
         case 'b': mode = COMPRESS_BST; break;
+        case 'p': mode = COMPRESS_PARALLEL; break;
         case 'd': mode = UNCOMPRESS; break;
         case 'r': report = 1; break;
         case 'i': use_index = 1; break;
@@ -92,16 +95,18 @@ int main(int argc, char *argv[])
             return EXIT_FAILURE;
         }
     }
+    const int codec_mode = mode == COMPRESS       ? SNAPPY_B200_MODE_HASH
+                           : mode == COMPRESS_BST ? SNAPPY_B200_MODE_BST
+                                                  : SNAPPY_B200_MODE_PARALLEL;
     const double t0 = now();
     if (framed && mode == UNCOMPRESS)
         rc = snappy_b200_frame_decompress_file(in, out);
     else if (framed)
-        rc = snappy_b200_frame_compress_file(in, out, mode == COMPRESS ? SNAPPY_B200_MODE_HASH : SNAPPY_B200_MODE_BST);
+        rc = snappy_b200_frame_compress_file(in, out, codec_mode);
     else if (idx && mode == UNCOMPRESS)
         rc = snappy_b200_decompress_file_indexed(in, idx, out);
-    else if (idx)
-        rc = snappy_b200_compress_file_indexed(in, in_size, mode == COMPRESS ? SNAPPY_B200_MODE_HASH : SNAPPY_B200_MODE_BST,
-                                               out, idx);
+    else if (idx || mode == COMPRESS_PARALLEL) /* (no index file: idx == NULL) */
+        rc = snappy_b200_compress_file_indexed(in, in_size, codec_mode, out, idx);
     else if (mode == COMPRESS)
         snappy_compress(in, in_size, out);
     else if (mode == COMPRESS_BST)

@@ -757,8 +757,12 @@ __global__ void __launch_bounds__(kEmitThreads) k_emit(const uint8_t *__restrict
 }
 
 // ------------------------------------------------------------------------------- launchers
+cudaError_t launch_parallel_parse(const uint8_t *, uint64_t, uint64_t, uint16_t *, uint8_t *, uint2 *, uint32_t *,
+                                  cudaStream_t, uint64_t *); // compress_parallel.cu
+
+// d_cand: SNAPPY_B200_MODE_PARALLEL's candidate offsets (a u16 per input byte); not used by the other modes.
 cudaError_t launch_compress(const uint8_t *d_in, uint64_t n_bytes, int mode, uint8_t *d_scratch, uint32_t *d_sizes,
-                            uint2 *d_recs, uint32_t *d_nrec, cudaStream_t st, uint64_t *launches)
+                            uint2 *d_recs, uint32_t *d_nrec, uint16_t *d_cand, cudaStream_t st, uint64_t *launches)
 {
     const uint64_t nb = (n_bytes + kBlock - 1) / kBlock;
     if (nb == 0)
@@ -781,6 +785,10 @@ cudaError_t launch_compress(const uint8_t *d_in, uint64_t n_bytes, int mode, uin
     if (mode == SNAPPY_B200_MODE_HASH) {
         k_parse_hash_global<<<(unsigned)chains, cta, 0, st>>>(d_in, n_bytes, nb, d_recs, d_nrec, d_scratch, counters);
         *launches += 1;
+    } else if (mode == SNAPPY_B200_MODE_PARALLEL) {
+        e = launch_parallel_parse(d_in, n_bytes, nb, d_cand, d_scratch, d_recs, d_nrec, st, launches);
+        if (e != cudaSuccess)
+            return e;
     } else {
         // exact mode: 8 Ki slots (16 KiB), then 64 Ki slots (128 KiB) for the blocks that outgrow them
         // (> 6144 distinct keys: text)

@@ -23,6 +23,7 @@
 
 namespace sb200 {
 int fail_msg(int code, const char *msg); // abi.cu: records the thread's last error
+int check_mode(int mode);                // abi.cu: SNAPPY_B200_OK, or SNAPPY_B200_ERR_ARG for an unknown mode
 void clear_error();
 int frame_compress_host_range(const void *, uint64_t, int, void *, uint64_t, uint64_t *, bool); // host_pipeline.cu
 int frame_decompress_buffer(const void *, uint64_t, void *, uint64_t, uint64_t *, bool);          // host_pipeline.cu
@@ -381,8 +382,9 @@ extern "C" {
 
 int snappy_b200_frame_compress_file(FILE *in, FILE *out, int mode)
 {
-    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
-        return sb200::fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
+    sb200::clear_error();
+    if (sb200::check_mode(mode) != SNAPPY_B200_OK)
+        return SNAPPY_B200_ERR_ARG;
     return compress_file(in, 0, out, mode, nullptr, true);
 }
 
@@ -390,6 +392,9 @@ int snappy_b200_frame_decompress_file(FILE *in, FILE *out) { return decompress_f
 
 int snappy_b200_compress_file_indexed(FILE *in, unsigned long long input_size, int mode, FILE *out, FILE *index_out)
 {
+    sb200::clear_error();
+    if (sb200::check_mode(mode) != SNAPPY_B200_OK)
+        return SNAPPY_B200_ERR_ARG;
     return compress_file(in, input_size, out, mode, index_out);
 }
 

@@ -37,7 +37,8 @@ int fail_msg(int code, const char *msg);
 void clear_error();
 int cuda_fail_msg(cudaError_t e, const char *what);
 int status_error(uint32_t st);
-size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed);
+size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed, int mode);
+int check_mode(int mode);
 void add_launches(uint64_t n);
 cudaError_t compress_chunk(const uint8_t *, uint64_t, uint64_t, int, bool, bool, uint8_t *, uint64_t, uint64_t *, uint32_t *,
                            void *, cudaStream_t);
@@ -511,7 +512,7 @@ static int compress_host_chunks(const void *in, uint64_t n_bytes, int mode, bool
     const uint64_t chunk = std::min<uint64_t>(kCompressChunk, align_up(n_bytes, kBlock));
     const uint64_t n_chunks = (n_bytes + chunk - 1) / chunk;
     const uint64_t out_cap_chunk = framed ? snappy_b200_frame_max_compressed_bytes(chunk) : max_compressed(chunk);
-    const size_t ws_bytes = compress_workspace_bytes_internal(chunk, framed);
+    const size_t ws_bytes = compress_workspace_bytes_internal(chunk, framed, mode);
     const int slots = (int)std::min<uint64_t>(kSlots, n_chunks);
     // buffers: s input, 4+s output, 8+s workspace, 12 small
     for (int s = 0; s < slots; ++s) {
@@ -614,8 +615,8 @@ int snappy_b200_compress_host_range(const void *in, uint64_t n_bytes, int mode, 
     clear_error();
     if (!out_bytes || (n_bytes && (!in || !out)))
         return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
-    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
-        return fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
+    if (check_mode(mode) != SNAPPY_B200_OK)
+        return SNAPPY_B200_ERR_ARG;
     *out_bytes = 0;
     if (n_bytes == 0)
         return SNAPPY_B200_OK; // reference: an empty input gives an empty stream
@@ -636,8 +637,8 @@ int frame_compress_host_range(const void *in, uint64_t n_bytes, int mode, void *
 {
     if (!out_bytes || !out || (n_bytes && !in))
         return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
-    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
-        return fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
+    if (check_mode(mode) != SNAPPY_B200_OK)
+        return SNAPPY_B200_ERR_ARG;
     *out_bytes = 0;
     int n_dev = 0;
     if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev < 1) { // no CPU path, also for the empty input

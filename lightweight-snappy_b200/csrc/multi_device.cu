@@ -25,7 +25,8 @@ int cuda_fail_msg(cudaError_t e, const char *what);
 int status_error(uint32_t st);
 void clear_error();
 void add_launches(uint64_t n);
-size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed);
+size_t compress_workspace_bytes_internal(uint64_t n_bytes, bool framed, int mode);
+int check_mode(int mode);
 cudaError_t compress_chunk(const uint8_t *, uint64_t, uint64_t, int, bool, bool, uint8_t *, uint64_t, uint64_t *, uint32_t *, void *,
                            cudaStream_t);
 const uint64_t *compress_chunk_offsets(void *, uint64_t);
@@ -144,8 +145,8 @@ int snappy_b200_compress_host_multi_range(const void *in, uint64_t n_bytes, int 
     clear_error();
     if (!out_bytes || (n_bytes && (!in || !out)))
         return fail_msg(SNAPPY_B200_ERR_ARG, "null pointer argument");
-    if (mode != SNAPPY_B200_MODE_HASH && mode != SNAPPY_B200_MODE_BST)
-        return fail_msg(SNAPPY_B200_ERR_ARG, "unknown mode");
+    if (check_mode(mode) != SNAPPY_B200_OK)
+        return SNAPPY_B200_ERR_ARG;
     *out_bytes = 0;
     if (n_bytes == 0)
         return SNAPPY_B200_OK;
@@ -181,7 +182,7 @@ int snappy_b200_compress_host_multi_range(const void *in, uint64_t n_bytes, int 
         W(a.init(), "arena init");
         W(a.need(0, 2 * chunk), "cudaMalloc");                                            // two input slots
         W(a.need(1, max_compressed(hi - lo) + 32 * n_chunks + 64), "cudaMalloc");        // all compressed chunks
-        W(a.need(2, compress_workspace_bytes_internal(chunk, false)), "cudaMalloc");
+        W(a.need(2, compress_workspace_bytes_internal(chunk, false, mode)), "cudaMalloc");
         W(a.need(3, 256), "cudaMalloc");
         uint8_t *d_in = static_cast<uint8_t *>(a.buf[0]);
         uint8_t *d_out = static_cast<uint8_t *>(a.buf[1]);
